@@ -68,7 +68,28 @@ def parse():
     ap.add_argument("--max-depth", type=int, default=16, help="developer knob (what the deep bounces cost); the benchmarked configuration is 16, the reference's default")
     ap.add_argument("--soup-rays", type=int, default=4096, help="soup workloads: the primary-ray grid is N x N (4096 -> 16.8 M rays)")
     ap.add_argument("--soup-builder", default="device", choices=["device", "host"], help="soup workloads: LBVH built on the device (csrc/lbvh.cuh) or the host binned-SAH builder")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path, default=None,
+                    help="after the timed steps, write what the last timed step computed to DIR/<name>.npy (a fixed sample of rows when the "
+                         "output is large), so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
+    return args
+
+
+def sample_rows(n, k):
+    """Indices of a fixed, seeded sample of k of n rows (all of them when n <= k), in ascending order."""
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+
+
+def dump_outputs(out_dir, arrays):
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out_dir / f"{name}.npy", a)
 
 
 def kernel_source_sha():
@@ -348,6 +369,10 @@ def main_gpu(args, wl):
         e1.record(stream)
         barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs is not None and rank == 0:
+        # the film accumulators of the last timed step, reduced onto rank 0; acc is reused by everything below
+        idx = torch.from_numpy(sample_rows(W * H, 1 << 20)).to(dev)
+        dump_outputs(args.dump_outputs, {"accumulators": acc.view(-1, 3)[idx].cpu().numpy()})
     ctx.set_option("stage_timing", 0)
     rays_mine = tot["closest_rays"] + tot["shadow_rays"]
     mx, sm = over_ranks([ms, rays_mine, tot["paths"], tot["kernel_launches"]])   # libtcpt's own kernels only: the ncclReduce kernel of a step is NCCL's
@@ -645,6 +670,20 @@ def soup_gpu(args, wl, world, rank, local):
         barrier()
         return a.elapsed_time(b) / steps
 
+    def hit_records(nn, any_hit):
+        """What tcpt_trace hands its caller for a fixed sample of the nn rays last traced into `hits`: {prim, tri, t, b0, b1, b2} per
+        closest hit (prim -1, the rest 0 for a miss), or the 0|1 flag of an any-hit ray (k_unpack_hits)."""
+        idx = torch.from_numpy(sample_rows(nn, 1 << 18)).to(dev)
+        tb = hits[: nn * 16].view(torch.float32).view(nn, 4)[idx].cpu().numpy().astype(np.float64)
+        pt = hits[nn * 16: nn * 24].view(torch.int32).view(nn, 2)[idx].cpu().numpy().astype(np.float64)
+        if any_hit:
+            return (pt[:, :1] >= 0).astype(np.float64)
+        rec = np.concatenate([pt, tb], 1)
+        rec[pt[:, 0] < 0, 1:] = 0.0
+        return rec
+
+    dump = args.dump_outputs is not None and rank == 0
+    outputs = {}
     o, d = soup_rays_numpy(args.soup_rays)
     n = len(o)
     rays_c = pack(o, d)
@@ -658,8 +697,15 @@ def soup_gpu(args, wl, world, rank, local):
     rays_i = pack(o2, d2)
     with ClockSampler(local, args.clock_period) as clk:
         ms_i = timed(rays_i, m, False, args.steps, args.warmup, hits)
+    if dump:
+        outputs["incoherent_closest"] = hit_records(m, False)
     ms_c = timed(rays_c, n, False, args.steps, args.warmup, hits)
+    if dump:
+        outputs["coherent_closest"] = hit_records(n, False)
     ms_s = timed(rays_i, m, True, args.steps, args.warmup, hits)
+    if dump:
+        outputs["incoherent_anyhit"] = hit_records(m, True)
+        dump_outputs(args.dump_outputs, outputs)
     counts = {}
     ctx.set_option("count_tests", 1)
     for name, (rr, nn, ah) in {"incoherent": (rays_i, m, False), "coherent": (rays_c, n, False), "anyhit": (rays_i, m, True)}.items():

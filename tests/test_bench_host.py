@@ -1,9 +1,13 @@
-"""bench.py's host-side logic (CPU-only): the reference arm runs without the product library, the CPU sample covers the whole frame,
-the profile digest is tied to the kernel sources it was captured from."""
+"""bench.py's host-side logic (CPU): the reference arm runs without the product library, the CPU sample covers the whole frame,
+the profile digest is tied to the kernel sources it was captured from, bad arguments are refused.  On the GPU: what --dump-outputs
+writes is the film of the last timed step."""
 import json
 import subprocess
 import sys
 from pathlib import Path
+
+import numpy as np
+import pytest
 
 ROOT = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(ROOT))
@@ -43,3 +47,31 @@ def test_profile_digest_names_the_kernel_sources_it_came_from():
     assert 150.0 <= s["dram_bytes"] / doc["closest_rays"] <= 400.0
     assert t["launches"] == 17 and t["fadd"] > 0 and t["fmul"] > 0
     assert len(bench.kernel_source_sha()) == 16
+
+
+def test_argument_checks():
+    for argv, msg in ((["--steps", "0"], "--steps must be at least 1"), (["--impl", "reference", "--dump-outputs", "out"], "--dump-outputs")):
+        r = subprocess.run([sys.executable, str(ROOT / "bench.py"), *argv], capture_output=True, text=True, timeout=120, cwd=str(ROOT))
+        assert r.returncode == 2 and msg in r.stderr, r.stderr[-2000:]
+
+
+def test_dump_sample_is_fixed():
+    a = bench.sample_rows(3840 * 2160, 1 << 20)
+    assert np.array_equal(a, bench.sample_rows(3840 * 2160, 1 << 20))
+    assert len(a) == 1 << 20 and np.all(np.diff(a) > 0) and a[-1] < 3840 * 2160
+    assert np.array_equal(bench.sample_rows(30000, 1 << 20), np.arange(30000))      # a small output is written whole
+
+
+@pytest.mark.gpu
+def test_dump_outputs_is_the_last_timed_step(bundle_factory, tmp_path):
+    """--steps 3 --warmup 1 at 4 sample indices per step: the timed steps are 1..3, the last one renders sample indices [12, 16)."""
+    r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--workload", "scene3_test", "--steps", "3", "--warmup", "1", "--spp-per-step", "4",
+                        "--no-cpu-baseline", "--no-extras", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600, cwd=str(ROOT))
+    assert r.returncode == 0, r.stderr[-2000:]
+    line = json.loads(r.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 3 and line["counts_rank0"]["paths"] == 3 * 200 * 150 * 4
+    assert sorted(p.name for p in tmp_path.iterdir()) == ["accumulators.npy"]
+    got = np.load(tmp_path / "accumulators.npy")
+    assert got.dtype == np.float32 and got.shape == (200 * 150, 3)
+    want = bundle_factory(3, 200, 150).image("mis", 512).render("sobol", spp_begin=12, spp_end=16).accumulators.reshape(-1, 3)
+    assert np.abs(got - want).max() <= 1e-5 * max(1.0, np.abs(want).max())

@@ -69,6 +69,7 @@ def _c_abi_shard(rank, world, mode, w, h, spp):
 
 
 def _worker(rank, world, port, mode, out_dir):
+    os.environ["CUDA_VISIBLE_DEVICES"] = ""      # a host-only rank on any machine: set before libtcpt initialises CUDA in this process
     sys.path.insert(0, str(ROOT))
     import torch
     import torch.distributed as dist
