@@ -148,6 +148,10 @@ struct DRender {
 };
 #define TCPT_SOBOL_HASH_N 512
 
+// An entry of the bucketed shading order: {queue position, path slot}.  The slot rides along so that the head of the path state is
+// asked for together with the ray and the hit record instead of after the ray has arrived (one round trip less in front of every vertex).
+typedef uint2 OrderEntry;
+
 // Wavefront buffers.  Path state is a structure of arrays of 16-byte records indexed by path slot; ray queues, hit records
 // and shadow queues are indexed by QUEUE POSITION so every stage reads and writes them fully coalesced.
 struct DState {
@@ -157,7 +161,7 @@ struct DState {
     float4* ext_o[2]; float4* ext_d[2];                     // {o.xyz, tmax} | {d.xyz, bits(slot)}   (ping-pong)
     float4* hit0; uint2* hit1;                              // {t, b0, b1, b2} | {prim, tri}
     float4* sh_o; float4* sh_d; float4* sh_c;               // shadow ray + pending NEE contribution (sh_d.w = slot | finalize << 31)
-    uint32_t* order; uint32_t capacity;                     // TCPT_N_BUCKETS x capacity queue positions, bucketed by shading work
+    OrderEntry* order; uint32_t capacity;                   // TCPT_N_BUCKETS x capacity order entries, bucketed by shading work
     uint32_t* counters;                                     // [0],[1] extension queue sizes (ping-pong), [2] shadow queue size,
                                                             // [4..10), [12..18) bucket sizes of even / odd bounces
     unsigned long long* stats;                              // [0] closest rays [1] shadow rays [2] box tests [3] tri tests [4] paths
@@ -242,27 +246,6 @@ struct DSampler {
         f.tables = R.sobol_prefix ? (R.prefix_dims | (R.pass_info << 16)) : 0u;
         f.cfg = R.log2_spp | (R.n_base4_digits << 8); f.seed = R.seed; f.hash_table = R.sobol_hash;
         return f;
-    }
-
-    // The table entries the next draws of this vertex will load (sample_index: one entry of the prefix table and one of the pass table per
-    // sampler call, each on its own 33 MB row: a DRAM round trip in front of every random number).  Their addresses only depend on the
-    // pixel and the dimension counter, so a vertex asks for them as soon as it knows both, long before the values are needed.
-#ifndef TCPT_PREFETCH_DRAWS
-#define TCPT_PREFETCH_DRAWS 0
-#endif
-    __device__ __forceinline__ void prefetch_draws(const DRender& R, uint32_t offsets) const {   // offsets: bit k set = a sampler call at dimension dim + k
-#if TCPT_PREFETCH_DRAWS
-        if (R.sampler != TCPT_SAMPLER_SOBOL || R.sobol_prefix == nullptr) return;
-        const uint32_t n_prefix = R.prefix_dims, n_pass = R.pass_info & 0xffu;
-        const uint32_t* col = R.sobol_prefix + pix;
-#pragma unroll
-        for (uint32_t k = 0; k < 8u; ++k) {
-            if (!((offsets >> k) & 1u)) continue;
-            const uint32_t d = dim + k;
-            if (d < n_prefix) asm volatile("prefetch.global.L2 [%0];" ::"l"(col + (size_t)d * R.prefix_stride));
-            if (d < n_pass) asm volatile("prefetch.global.L2 [%0];" ::"l"(col + (size_t)(n_prefix + d) * R.prefix_stride));
-        }
-#endif
     }
 
     __device__ __forceinline__ static uint32_t perm_digit(uint32_t p, uint32_t digit) {
@@ -414,33 +397,6 @@ struct DSampler {
         }
         return r;
     }
-    // the same with the lobe choice in front (a 1-D call at dimension d0): what the other material buckets draw on their usual way through a vertex
-    struct Draws4 { float2 a, b; float c, u0; };
-    __device__ __noinline__ static Draws4 sobol_draws4(uint32_t morton, uint32_t d0, uint32_t da, uint32_t db, uint32_t dc, uint32_t pix, const SobolFrame f) {
-        const SobolLoads l0 = sample_index_loads(d0, pix, f), la = sample_index_loads(da, pix, f), lb = sample_index_loads(db, pix, f), lc = sample_index_loads(dc, pix, f);
-        Draws4 r;
-        {
-            const uint64_t a = sample_index_from(morton, d0, f, l0);
-            r.u0 = to_unit(owen(__brev((uint32_t)a), (uint32_t)hash_of(d0 + 1u, f)));
-        }
-        {
-            const uint64_t a = sample_index_from(morton, da, f, la);
-            const uint64_t h = hash_of(da + 2u, f);
-            r.a.x = to_unit(owen(__brev((uint32_t)a), (uint32_t)h));
-            r.a.y = to_unit(owen(sobol_dim1(a), (uint32_t)(h >> 32)));
-        }
-        {
-            const uint64_t a = sample_index_from(morton, db, f, lb);
-            const uint64_t h = hash_of(db + 2u, f);
-            r.b.x = to_unit(owen(__brev((uint32_t)a), (uint32_t)h));
-            r.b.y = to_unit(owen(sobol_dim1(a), (uint32_t)(h >> 32)));
-        }
-        {
-            const uint64_t a = sample_index_from(morton, dc, f, lc);
-            r.c = to_unit(owen(__brev((uint32_t)a), (uint32_t)hash_of(dc + 1u, f)));
-        }
-        return r;
-    }
     // get_1d whose value the caller provably does not use: both samplers are pure functions of the dimension counter, so
     // advancing the counter is all that has to happen (the reference computes and discards the value)
     __device__ __forceinline__ void skip_1d() { dim += 1; }
@@ -503,9 +459,6 @@ __device__ __forceinline__ float4 cmf_at(const DScene& sc, float lambda) {  // D
     return i < 470u ? __ldg(&sc.cmf[i]) : make_float4(0, 0, 0, 0);
 }
 
-#ifndef TCPT_ILLUM_HALF
-#define TCPT_ILLUM_HALF 1
-#endif
 // RgbToSpectrumTable::get (rgb_sigmoid_polynomial.rs:87-155), sRGB-gamma typed colour
 // (returns by value: an out-array lived in local memory and cost a store -> load -> store -> load chain through L1 before the first
 // wavelength could be evaluated)
@@ -602,7 +555,7 @@ __device__ __forceinline__ DSpectrum illuminant_from_rgb(const DScene& sc, float
     DSpectrum s; s.kind = 2; s.table = 0;
     const float mx = rmax(rgb.x, rmax(rgb.y, rgb.z));
     s.scale = 2.0f * mx;
-    const float3 c = rgb_to_coeffs_t<TCPT_ILLUM_HALF != 0>(sc, rgb / s.scale);
+    const float3 c = rgb_to_coeffs_t<true>(sc, rgb / s.scale);
     s.c[0] = c.x; s.c[1] = c.y; s.c[2] = c.z;
     return s;
 }
@@ -666,24 +619,6 @@ __device__ __forceinline__ void warp_push2(uint32_t* ca, bool pa, uint32_t* cb, 
     const uint32_t ba = __shfl_sync(0xffffffffu, base, 0), bb = __shfl_sync(0xffffffffu, base, 1);
     const uint32_t below = (1u << lane) - 1u;
     *ia = ba + (uint32_t)__popc(ma & below); *ib = bb + (uint32_t)__popc(mb & below);
-}
-// the same in two halves: begin issues the two atomics and does not wait for them, end hands out the positions.  What the caller puts
-// between the two (the loads of its next vertex) overlaps the atomics' round trip.
-struct Push2 { uint32_t ma, mb, base; };
-__device__ __forceinline__ Push2 warp_push2_begin(uint32_t* ca, bool pa, uint32_t* cb, bool pb) {
-    Push2 t;
-    t.ma = __ballot_sync(0xffffffffu, pa); t.mb = __ballot_sync(0xffffffffu, pb);
-    const uint32_t lane = threadIdx.x & 31u;
-    t.base = 0;
-    if (lane == 0u) { if (t.ma) t.base = atomicAdd(ca, (uint32_t)__popc(t.ma)); }
-    else if (lane == 1u) { if (t.mb) t.base = atomicAdd(cb, (uint32_t)__popc(t.mb)); }
-    return t;
-}
-__device__ __forceinline__ void warp_push2_end(const Push2& t, uint32_t* ia, uint32_t* ib) {
-    const uint32_t lane = threadIdx.x & 31u;
-    const uint32_t ba = __shfl_sync(0xffffffffu, t.base, 0), bb = __shfl_sync(0xffffffffu, t.base, 1);
-    const uint32_t below = (1u << lane) - 1u;
-    *ia = ba + (uint32_t)__popc(t.ma & below); *ib = bb + (uint32_t)__popc(t.mb & below);
 }
 // warp-aggregated queue append: every lane of the warp must call it (pred = false for lanes with nothing to push)
 __device__ __forceinline__ uint32_t warp_push(uint32_t* counter, bool pred) {

@@ -26,25 +26,14 @@
 #pragma once
 #include "dcommon.cuh"
 
-#ifndef TCPT_SORT_FULL
-#define TCPT_SORT_FULL 1          // 1: the hit children of a wide node are visited nearest first, the rest pushed far to near; 0: nearest first, rest unordered
-#endif
-#ifndef TCPT_BOTH_PHASES
-#define TCPT_BOTH_PHASES 0       // 1: no phase vote, every iteration runs a triangle step for the lanes holding triangles and a walking step for the others
-#endif
 #ifndef TCPT_MIN_CHUNK
 #define TCPT_MIN_CHUNK 32         // smallest block of ray indices a warp reserves at a time
 #endif
 static_assert(TCPT_MIN_CHUNK >= 32, "a refill hands the idle lanes of a warp consecutive indices of ONE chunk: it must cover a whole warp");
-#ifndef TCPT_ANYHIT_UNSORTED
-#define TCPT_ANYHIT_UNSORTED 1
-#endif
-#ifndef TCPT_POP_CULL
-#define TCPT_POP_CULL 1           // closest hit: a stack entry carries the entry distance of its box and is dropped when it comes off the stack behind the best hit
-#endif
 #ifndef TCPT_SMEM_STACK
 #define TCPT_SMEM_STACK 8         // the SHORT stack: the first 8 traversal-stack entries live in shared memory (one word per thread and row), deeper ones spill to local memory (measured 0 / 8 / 16 entries: 29.87 / 29.76 / 30.2 ms of traversal per step)
 #endif
+static_assert(TCPT_SMEM_STACK > 0, "the traversal stack keeps its first entries in shared memory");
 
 namespace tcpt {
 
@@ -177,12 +166,8 @@ enum {
 };
 struct TraceShared {
     uint32_t w[TS_WORDS][128];
-#if TCPT_SMEM_STACK > 0
     uint32_t stack[TCPT_SMEM_STACK][128];
-#if TCPT_POP_CULL
     float stack_t[TCPT_SMEM_STACK][128];
-#endif
-#endif
 };
 #define TS_F(row) __uint_as_float(S.w[row][tid])
 #define TS_U(row) S.w[row][tid]
@@ -215,44 +200,23 @@ struct Traversal {
     }
     __device__ __forceinline__ bool holds_triangles() const { return (cur & TCPT_ENTRY_LEAF) != 0u && blas_sp >= 0; }   // (cur is never NONE between steps)
 
-    // A stack entry of a closest-hit walk carries the entry distance `te` of its box (TCPT_POP_CULL): see advance().
+    // A stack entry of a closest-hit walk carries the entry distance `te` of its box: see advance().
     template <bool ANY>
     __device__ __forceinline__ void push(TraceShared& S, uint32_t tid, uint32_t* stack, float* stack_t, uint32_t v, float te) {
-#if TCPT_SMEM_STACK > 0
         if (sp < TCPT_SMEM_STACK) {
             S.stack[sp][tid] = v;
-#if TCPT_POP_CULL
             if (!ANY) S.stack_t[sp][tid] = te;
-#endif
         } else {
             stack[sp - TCPT_SMEM_STACK] = v;
-#if TCPT_POP_CULL
             if (!ANY) stack_t[sp - TCPT_SMEM_STACK] = te;
-#endif
         }
         ++sp;
-#else
-        stack[sp] = v;
-#if TCPT_POP_CULL
-        if (!ANY) stack_t[sp] = te;
-#endif
-        ++sp;
-#endif
     }
     template <bool ANY>
     __device__ __forceinline__ uint32_t pop(TraceShared& S, uint32_t tid, uint32_t* stack, float* stack_t, float* te) {
         --sp;
-#if TCPT_SMEM_STACK > 0
-#if TCPT_POP_CULL
         if (!ANY) *te = sp < TCPT_SMEM_STACK ? S.stack_t[sp][tid] : stack_t[sp - TCPT_SMEM_STACK];
-#endif
         return sp < TCPT_SMEM_STACK ? S.stack[sp][tid] : stack[sp - TCPT_SMEM_STACK];
-#else
-#if TCPT_POP_CULL
-        if (!ANY) *te = stack_t[sp];
-#endif
-        return stack[sp];
-#endif
     }
 
     // Tests the first triangle of the pending leaf range.  ANY = Scene::intersect_p (scene.rs:93-103): returns true (ray finished) at the first accepted triangle.
@@ -343,17 +307,15 @@ struct Traversal {
             h3 = ent.w != TCPT_ENTRY_NONE && slab_exact(lx.w, ly.w, lz.w, hx.w, hy.w, hz.w, r, limit, &te3);
         }
         if (COUNT) (*n_box) += (ent.x != TCPT_ENTRY_NONE) + (ent.y != TCPT_ENTRY_NONE) + (ent.z != TCPT_ENTRY_NONE) + (ent.w != TCPT_ENTRY_NONE);
-        // order the hit children by entry distance (misses sort last)
+        // order the hit children by entry distance (misses sort last): the nearest is visited next, the others are pushed far to near
         float k0 = h0 ? te0 : TCPT_INF, k1 = h1 ? te1 : TCPT_INF, k2 = h2 ? te2 : TCPT_INF, k3 = h3 ? te3 : TCPT_INF;
         uint32_t e0 = h0 ? ent.x : TCPT_ENTRY_NONE, e1 = h1 ? ent.y : TCPT_ENTRY_NONE, e2 = h2 ? ent.z : TCPT_ENTRY_NONE, e3 = h3 ? ent.w : TCPT_ENTRY_NONE;
 #define TCPT_CE(ka, ea, kb, eb) { const bool sw = kb < ka; const float kt = sw ? kb : ka; kb = sw ? ka : kb; ka = kt; const uint32_t et = sw ? eb : ea; eb = sw ? ea : eb; ea = et; }
         // (any hit: the answer does not depend on the order of the walk, and a ray that reaches its light -- most do -- visits every box it
         // passes whatever the order: no ordering network)
-        if (!ANY || !TCPT_ANYHIT_UNSORTED) {
+        if (!ANY) {
             TCPT_CE(k0, e0, k1, e1) TCPT_CE(k2, e2, k3, e3) TCPT_CE(k0, e0, k2, e2)
-#if TCPT_SORT_FULL
             TCPT_CE(k1, e1, k3, e3) TCPT_CE(k1, e1, k2, e2)
-#endif
         }
 #undef TCPT_CE
         if (e3 != TCPT_ENTRY_NONE) push<ANY>(S, tid, stack, stack_t, e3, k3);
@@ -367,7 +329,7 @@ struct Traversal {
     // or a triangle at hand -- or is finished NOW: with nothing at hand, the ray is done when the stack is empty; a stack back at
     // its height of BLAS entry means this instance is exhausted (back to the Render-space ray); otherwise the next entry comes off.
     // (As separate walking steps these cost every ray one or two of its five or so iterations: rays here are short.)
-    // Closest hit (TCPT_POP_CULL): an entry whose box is entered behind the culling bound is dropped as it comes off the stack.  The bound has
+    // Closest hit: an entry whose box is entered behind the culling bound is dropped as it comes off the stack.  The bound has
     // shrunk since the entry was pushed; every box below it is entered at or behind its own entry distance (the slab test is monotone
     // in the box, see the header), so the visit would have failed all of its slab tests: same candidates, one wide-node visit (or one
     // instance transform plus the visit of the BLAS root) less.
@@ -384,7 +346,7 @@ struct Traversal {
             }
             float te = 0.0f;
             cur = pop<ANY>(S, tid, stack, stack_t, &te);
-            if (ANY || !TCPT_POP_CULL || !(te > limit)) return false;
+            if (ANY || !(te > limit)) return false;
         }
     }
 };
@@ -398,9 +360,6 @@ struct Traversal {
 #define TCPT_TRI_PHASE_LANES 8    // a warp runs a triangle iteration once this many lanes hold pending triangles (4 / 8 / 12: 31.4 / 30.4 / 30.9 ms; no vote at all, both phases every iteration: 31.2)
 #endif
 #define TCPT_LOCAL_STACK (TCPT_TRAVERSAL_STACK - TCPT_SMEM_STACK)
-#ifndef TCPT_SPLIT_COMMIT
-#define TCPT_SPLIT_COMMIT 1       // a commit is begun (its loads and its atomic issued) before the refill asks for the next rays and ended after: the round trips overlap (measured neutral: 29.68 vs 29.66 ms; the kernel is bound by instruction issue, not by these waits)
-#endif
 
 // What a finished ray leaves behind, in two halves around the refill's ray loads: begin() issues the loads / the atomic whose results
 // end() needs (ncu: the shuffle waiting for the bucket counter's atomic and the first use of the freshly loaded ray were the two top stall
@@ -424,11 +383,7 @@ __device__ __forceinline__ void trace_queue(const DScene& sc, TraceShared& S, co
     const uint32_t FULL = 0xffffffffu, NONE = 0xffffffffu;
     const uint32_t lane = threadIdx.x & 31u, tid = threadIdx.x;
     uint32_t stack[TCPT_LOCAL_STACK];
-#if TCPT_POP_CULL
     float stack_t[ANY ? 1 : TCPT_LOCAL_STACK];
-#else
-    float stack_t[1];
-#endif
     Traversal T;
     T.cur = TCPT_ENTRY_NONE; T.blas_sp = -1;
     uint32_t ray = NONE, fin = NONE;
@@ -451,14 +406,9 @@ __device__ __forceinline__ void trace_queue(const DScene& sc, TraceShared& S, co
         const bool committing = fin != NONE;
         if (committing) {
             DHit h; T.result(S, tid, h); tok = commit.begin(fin, h); fin = NONE;
-#if !TCPT_SPLIT_COMMIT
-            commit.end(tok);
-#endif
         }
-#if TCPT_SPLIT_COMMIT
         float4 new_o = make_float4(0.0f, 0.0f, 0.0f, 0.0f), new_d = new_o;
         uint32_t mine = NONE;
-#endif
         if (n_idle != 0u) {
             uint32_t base_b = 0;
             if (fetch) {
@@ -468,31 +418,18 @@ __device__ __forceinline__ void trace_queue(const DScene& sc, TraceShared& S, co
             if (ray == NONE) {
                 // the first `left` idle lanes take what remains of the old chunk, the others start the new one
                 const uint32_t rk = (uint32_t)__popc(idle & ((1u << lane) - 1u));
-#if TCPT_SPLIT_COMMIT
                 if (rk < left) mine = pool + rk;
                 else if (fetch) mine = base_b + (rk - left);
                 if (mine < n) { new_o = q_o[mine]; new_d = q_d[mine]; }
-#else
-                uint32_t mine = NONE;
-                if (rk < left) mine = pool + rk;
-                else if (fetch) mine = base_b + (rk - left);
-                if (mine < n) {
-                    const float4 o = q_o[mine], d = q_d[mine];
-                    T.init(S, tid, f3(o.x, o.y, o.z), f3(d.x, d.y, d.z), o.w);
-                    ray = mine;
-                }
-#endif
             }
             if (fetch) { pool = base_b + (n_idle - left); pool_end = base_b + chunk; if (pool_end > n) pool_end = n; if (pool > pool_end) pool = pool_end; }
             else { pool += n_idle; if (pool > pool_end) pool = pool_end; }
         }
-#if TCPT_SPLIT_COMMIT
         if (committing) commit.end(tok);
         if (mine < n) {   // (mine == NONE for a lane that did not refill)
             T.init(S, tid, f3(new_o.x, new_o.y, new_o.z), f3(new_d.x, new_d.y, new_d.z), new_o.w);
             ray = mine;
         }
-#endif
         const bool exhausted = drained && pool >= pool_end;
         if (__ballot_sync(FULL, ray != NONE) == 0u) break;  // nothing in flight and nothing left to fetch
         const uint32_t stop_at = exhausted ? 32u : refill_lanes;
@@ -500,12 +437,6 @@ __device__ __forceinline__ void trace_queue(const DScene& sc, TraceShared& S, co
         do {
             const bool has_tri = ray != NONE && T.holds_triangles();
             const bool walks = ray != NONE && !has_tri;
-#if TCPT_BOTH_PHASES
-            // no vote: the lanes holding triangles test one, then the walking lanes visit a node, every iteration
-            bool finished = false;
-            if (has_tri) finished = T.template tri_step<ANY, COUNT>(sc, S, tid, stack, stack_t, n_tri);
-            if (walks) finished = T.template node_step<ANY, COUNT>(sc, S, tid, stack, stack_t, n_box);
-#else
             const uint32_t tri_mask = __ballot_sync(FULL, has_tri);
             const uint32_t node_mask = __ballot_sync(FULL, walks);
             bool finished = false;
@@ -514,7 +445,6 @@ __device__ __forceinline__ void trace_queue(const DScene& sc, TraceShared& S, co
             } else {
                 if (walks) finished = T.template node_step<ANY, COUNT>(sc, S, tid, stack, stack_t, n_box);
             }
-#endif
             if (finished) { fin = ray; ray = NONE; T.cur = TCPT_ENTRY_NONE; }
             n_idle_now = (uint32_t)__popc(__ballot_sync(FULL, ray == NONE));
         } while (n_idle_now < stop_at);

@@ -22,33 +22,8 @@
 #define TCPT_TRACE_MIN_BLOCKS 8   // 64 registers + 13 KB of shared memory per block: 32 warps per SM (measured 6 / 7 / 8 blocks: 35.7 / 33.5 / 32.1 ms per step)
 #endif
 #define TCPT_BUCKET_STRIDE 10
-#ifndef TCPT_SPLIT_PUSH
-#define TCPT_SPLIT_PUSH 0    // 1: the queue-append atomics of a vertex are issued, then the loads of the thread's next vertex, then the rays are stored.  Measured slower (31.73 vs 31.47 ms of shading per step): the 20 words of the pending rays stay live across the next vertex's loads
-#endif
-#ifndef TCPT_PBR_DRAWS4
-#define TCPT_PBR_DRAWS4 0    // 1: the other material buckets draw their four sampler calls at once (sobol_draws4).  Measured slower on scene 19 (31.52 vs 30.98 ms of shading per step: six more live values in kernels that already spill), neutral on scene 17
-#endif
-#ifndef TCPT_LAMBERT_DRAWS3
-#define TCPT_LAMBERT_DRAWS3 1
-#endif
-#ifndef TCPT_ORDER_SLOT
-#define TCPT_ORDER_SLOT 1    // an entry of the bucketed order is {queue position, path slot} (8 B) instead of the queue position alone
-#endif
-#ifndef TCPT_ORDER_AHEAD
-#define TCPT_ORDER_AHEAD 1   // the order entry of a thread's NEXT vertex is loaded before the current one is shaded
-#endif
 
 namespace tcpt {
-
-// TCPT_ORDER_SLOT: an order entry carries the path slot next to the queue position, so the head of the path state is asked for together
-// with the ray and the hit record instead of after the ray has arrived (one round trip less in front of every vertex).
-#if TCPT_ORDER_SLOT
-typedef uint2 OrderEntry;
-__device__ __forceinline__ OrderEntry make_order(uint32_t i, uint32_t slot) { return make_uint2(i, slot); }
-#else
-typedef uint32_t OrderEntry;
-__device__ __forceinline__ OrderEntry make_order(uint32_t i, uint32_t) { return i; }
-#endif
 
 struct PathList { const uint32_t* xy; const uint32_t* sample; };  // explicit (pixel, sample) lists for tcpt_path_samples
 
@@ -264,7 +239,7 @@ struct CommitClosest {
     __device__ __forceinline__ void end(const CommitToken& t) const {
         const uint32_t lane = threadIdx.x & 31u, peers = t.b, b = t.c, i = t.d;
         const uint32_t base = __shfl_sync(peers, t.a, __ffs(peers) - 1);
-        ((OrderEntry*)st.order)[(size_t)b * st.capacity + base + (uint32_t)__popc(peers & ((1u << lane) - 1u))] = make_order(i, t.e);
+        st.order[(size_t)b * st.capacity + base + (uint32_t)__popc(peers & ((1u << lane) - 1u))] = make_uint2(i, t.e);
     }
 };
 // what a finished shadow ray does: add the pending NEE contribution if the light is visible (common.rs:134-170); hand a path that
@@ -379,19 +354,14 @@ __device__ __forceinline__ void shade_vertex(const DScene& sc, const DRender& R,
     smp.dim = __float_as_uint(misc.z);
     // sampler calls of one bounce sit at dimension offsets 0 (lobe choice; Lambert and metal skip it), 1 (direction), 3 (light choice, skipped
     // with one light), 4 (triangle of an area light), 5 (point on the light) and 7 (Russian roulette; 3 under pt, which draws nothing for lights)
-    if (!BucketInfo<B>::miss && !BucketInfo<B>::terminal && MT != TCPT_MAT_EMISSIVE)
-        smp.prefetch_draws(R, ((MT == TCPT_MAT_LAMBERT || MT == TCPT_MAT_METAL) ? 0u : 1u) | 2u | (R.integrator != TCPT_INTEGRATOR_PT ? 0xa0u : 0x08u));
     // Lambert under nee / mis with the Sobol sampler: the direction, the point on the light and Russian roulette sit at dimension offsets 1, 5
     // and 7 on the usual way through the vertex; all three are drawn here in one call (DSampler::sobol_draws3) and handed out below if the
     // dimension counter is where it was expected to be (otherwise the ordinary call runs: same values either way)
     constexpr bool NO_LOBE = MT == TCPT_MAT_LAMBERT || MT == TCPT_MAT_METAL;   // these never read the lobe-choice number
-    constexpr bool PRE = !BucketInfo<B>::miss && !BucketInfo<B>::terminal && MT != TCPT_MAT_EMISSIVE && (MT == TCPT_MAT_LAMBERT ? TCPT_LAMBERT_DRAWS3 != 0 : TCPT_PBR_DRAWS4 != 0);
-    DSampler::Draws4 pre; bool have_pre = false; const uint32_t pre_d0 = smp.dim;
+    constexpr bool PRE = MT == TCPT_MAT_LAMBERT;
+    DSampler::Draws3 pre; bool have_pre = false; const uint32_t pre_d0 = smp.dim;
     if (PRE && R.sampler == TCPT_SAMPLER_SOBOL && R.integrator != TCPT_INTEGRATOR_PT && (FIRST || stage < R.max_depth)) {
-        if (NO_LOBE) {
-            const DSampler::Draws3 t = DSampler::sobol_draws3(smp.morton, pre_d0 + 1u, pre_d0 + 5u, pre_d0 + 7u, smp.pix, DSampler::frame_of(R));
-            pre.a = t.a; pre.b = t.b; pre.c = t.c; pre.u0 = 0.0f;
-        } else pre = DSampler::sobol_draws4(smp.morton, pre_d0, pre_d0 + 1u, pre_d0 + 5u, pre_d0 + 7u, smp.pix, DSampler::frame_of(R));
+        pre = DSampler::sobol_draws3(smp.morton, pre_d0 + 1u, pre_d0 + 5u, pre_d0 + 7u, smp.pix, DSampler::frame_of(R));
         have_pre = true;
     }
     S4 thr = s4(1.0f), con = s4(0.0f);
@@ -504,7 +474,6 @@ __device__ __forceinline__ void shade_vertex(const DScene& sc, const DRender& R,
     // `uc` only selects between lobes; LambertMaterial::sample and MetalMaterial::sample never read it (lambert_material.rs:42-97, metal_material.rs:124)
     float uc = 0.0f;
     if (NO_LOBE) smp.skip_1d();
-    else if (PRE && have_pre && smp.dim == pre_d0) { uc = pre.u0; smp.dim += 1; }
     else uc = smp.get_1d(R);
     float2 uv;
     if (PRE && have_pre && smp.dim == pre_d0 + 1u) { uv = pre.a; smp.dim += 2; } else uv = smp.get_2d(R);
@@ -682,12 +651,12 @@ __device__ __forceinline__ void shade_vertex(const DScene& sc, const DRender& R,
 
 // What a vertex reads before it can start: its queue position (through the bucketed order), the ray it arrived on, the hit record and
 // the head of its path state: a chain of DEPENDENT loads (order -> ray -> slot -> state), each a DRAM round trip at the benchmarked pass
-// size.  The order entry of the NEXT vertex is asked for before this one is shaded (one or two registers across the vertex).
+// size.  The order entry of the NEXT vertex is asked for before this one is shaded (two registers across the vertex).
 struct VertexIn { float4 d, h0, misc; uint2 h1; };
 template <int B>
 __device__ __forceinline__ OrderEntry load_order(const DState& st, uint32_t p, uint32_t n) {
-    OrderEntry o = make_order(0u, 0u);
-    if (p < n) o = ((const OrderEntry*)st.order)[(size_t)B * st.capacity + p];
+    OrderEntry o = make_uint2(0u, 0u);
+    if (p < n) o = st.order[(size_t)B * st.capacity + p];
     return o;
 }
 template <int B>
@@ -695,37 +664,18 @@ __device__ __forceinline__ VertexIn load_vertex(const DState& st, int cur, Order
     VertexIn v;
     v.d = make_float4(0.0f, 0.0f, 0.0f, 0.0f); v.h0 = v.d; v.misc = v.d; v.h1 = make_uint2(0u, 0u);
     if (valid) {
-#if TCPT_ORDER_SLOT
         const uint32_t i = o.x;
         v.misc = st.misc[o.y];
         v.d = st.ext_d[cur][i];
-#else
-        const uint32_t i = o;
-        v.d = st.ext_d[cur][i];
-#endif
         if (B < 7) { v.h0 = st.hit0[i]; v.h1 = st.hit1[i]; }   // an escaped ray and a path Russian roulette ended read nothing of the hit record: 24 B per vertex less
-#if !TCPT_ORDER_SLOT
-        v.misc = st.misc[__float_as_uint(v.d.w) & 0x7fffffffu];
-#endif
     }
     return v;
 }
-// Shades position p of bucket B's range of the bucketed order (p >= n: the lane only takes part in the warp-collective pushes).  In two
-// halves: shade_position_begin shades the vertex and ISSUES the two queue-append atomics, shade_position_end waits for them and stores the
-// rays; the kernel asks for its next vertex in between, so that the atomics' round trip and the next vertex's loads overlap.
-struct ShadePending { ShadeOut out; Push2 push; };
-template <int B, bool FIRST = false>
-__device__ __forceinline__ void shade_position_begin(const DScene& sc, const DRender& R, const DState& st, const PathList& L, int cur, int sh, uint32_t stage, uint32_t p, uint32_t n, const VertexIn& v, ShadePending& pend) {
-    pend.out.push_ext = false; pend.out.push_sh = false;
-    if (p < n) shade_vertex<B, FIRST>(sc, R, st, L, stage, f3(v.d.x, v.d.y, v.d.z), __float_as_uint(v.d.w) & 0x7fffffffu, v.h0, v.h1, v.misc, pend.out);
-    if (B < 6) pend.push = warp_push2_begin(&st.counters[cur ^ 1], pend.out.push_ext, &st.counters[sh], pend.out.push_sh);   // emissive hits and misses end the path: nothing to push
-}
-template <int B>
-__device__ __forceinline__ void shade_position_end(const DState& st, int cur, const ShadePending& pend) {
-    if (B < 6) {
+// Appends the extension and shadow rays a vertex of bucket b spawned to their queues.  Every lane of the warp must call it with the same b.
+__device__ __forceinline__ void push_rays(const DState& st, int cur, int sh, int b, const ShadeOut& out) {
+    if (b < 6) {   // emissive hits and misses end the path: nothing to push
         uint32_t pe, ps;
-        warp_push2_end(pend.push, &pe, &ps);
-        const ShadeOut& out = pend.out;
+        warp_push2(&st.counters[cur ^ 1], out.push_ext, &st.counters[sh], out.push_sh, &pe, &ps);
         if (out.push_ext) { st.ext_o[cur ^ 1][pe] = out.eo; st.ext_d[cur ^ 1][pe] = out.ed; }
         if (out.push_sh) { st.sh_o[ps] = out.so; st.sh_d[ps] = out.sd; st.sh_c[ps] = out.sc; }
     }
@@ -744,12 +694,6 @@ __device__ __forceinline__ void shade_position_end(const DState& st, int cur, co
 #ifndef TCPT_SHADE_MIN_BLOCKS_MISS
 #define TCPT_SHADE_MIN_BLOCKS_MISS 8                 // their resident 128-thread units per SM (8: 64 registers).  256-thread blocks x 3 (85 registers, no spills) / x 4, 128-thread blocks x 5: 31.5 / 31.4 / 32.4 ms of shading per step against 31.4 (profiles/r02l_ab_miss_bucket_configs.log)
 #endif
-#ifndef TCPT_SHADE_SYNC
-#define TCPT_SHADE_SYNC 1
-#endif
-#ifndef TCPT_SHADE_PIPELINE
-#define TCPT_SHADE_PIPELINE 0   // 1: issue the loads of the NEXT vertex before shading this one.  Measured slower (34.3 vs 32.8 ms of shading per step): the 15 registers it holds across the vertex cost more than the four round trips it hides
-#endif
 // block shape of k_shade<B>: the material buckets run ONE big block per SM whose warps start every vertex together (see the kernel);
 // the register budget follows from the block size (512 threads: 128 registers, 640: 96, 768: 80)
 template <int B> struct ShadeCfg {
@@ -763,38 +707,23 @@ __global__ void __launch_bounds__(ShadeCfg<B>::threads, ShadeCfg<B>::min_blocks)
     if (B == 0 && blockIdx.x == 0 && threadIdx.x == 0) { st.counters[24] = 0; st.counters[25] = 0; }  // work counters of the next trace launch
     const uint32_t stride = gridDim.x * blockDim.x;
     const uint32_t n = st.counters[4 + TCPT_BUCKET_STRIDE * cur + B];
-    // whole warps iterate together (warp_push is warp-collective); with TCPT_SHADE_SYNC whole blocks do, and start every vertex together
-    const uint32_t unit = (TCPT_SHADE_SYNC && B < 6) ? (uint32_t)ShadeCfg<B>::threads : 32u;
+    // whole warps iterate together (push_rays is warp-collective); in the material buckets whole blocks do, and start every vertex together
+    const uint32_t unit = B < 6 ? (uint32_t)ShadeCfg<B>::threads : 32u;
     const uint32_t n_round = (n + unit - 1u) / unit * unit;
-    // software pipeline: the loads of the NEXT vertex are issued before this one is shaded, so their round trips overlap the shading
-    // instead of standing in front of it (ncu: 15 % of the Lambert kernel's stall samples sat on these four loads)
+    // the order entry of the NEXT vertex is loaded before this one is shaded: of the dependent round trips in front of a vertex only one
+    // is left exposed (ncu: 15 % of the Lambert kernel's stall samples sat on these loads).  Loading the whole next vertex ahead holds
+    // 15 registers across the shading and was slower (DESIGN.md section 3).
     uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
     VertexIn v = load_vertex<B>(st, cur, load_order<B>(st, p, n), p < n);
     for (; p < n_round; p += stride) {
         const uint32_t pn = p + stride;
         const bool more = pn < n && pn > p;
-#if TCPT_ORDER_AHEAD
         const OrderEntry o_next = load_order<B>(st, pn, more ? n : 0u);
-#endif
-#if TCPT_SHADE_PIPELINE
-        const VertexIn next = load_vertex<B>(st, cur, load_order<B>(st, pn, more ? n : 0u), more);
-#endif
-        if (TCPT_SHADE_SYNC && B < 6) __syncthreads();
-        ShadePending pend;
-        shade_position_begin<B, FIRST>(sc, R, st, L, cur, sh, stage, p, n, v, pend);
-#if !TCPT_SPLIT_PUSH
-        shade_position_end<B>(st, cur, pend);
-#endif
-#if TCPT_SHADE_PIPELINE
-        v = next;
-#elif TCPT_ORDER_AHEAD
+        if (B < 6) __syncthreads();
+        ShadeOut out; out.push_ext = false; out.push_sh = false;   // (p >= n: the lane only takes part in the warp-collective push)
+        if (p < n) shade_vertex<B, FIRST>(sc, R, st, L, stage, f3(v.d.x, v.d.y, v.d.z), __float_as_uint(v.d.w) & 0x7fffffffu, v.h0, v.h1, v.misc, out);
+        push_rays(st, cur, sh, B, out);
         v = load_vertex<B>(st, cur, o_next, more);
-#else
-        v = load_vertex<B>(st, cur, load_order<B>(st, pn, more ? n : 0u), more);
-#endif
-#if TCPT_SPLIT_PUSH
-        shade_position_end<B>(st, cur, pend);
-#endif
     }
 }
 
@@ -824,11 +753,7 @@ __global__ void __launch_bounds__(128, TCPT_SHADE_MIN_BLOCKS) k_shade_all(const 
         const uint32_t p = c * 128u + threadIdx.x;
         ShadeOut out; out.push_ext = false; out.push_sh = false;
         if (p < n) {
-#if TCPT_ORDER_SLOT
-            const uint32_t i = ((const OrderEntry*)st.order)[(size_t)b * st.capacity + p].x;
-#else
-            const uint32_t i = st.order[(size_t)b * st.capacity + p];
-#endif
+            const uint32_t i = st.order[(size_t)b * st.capacity + p].x;
             switch (b) {
                 case 0: shade_vertex_call<0>(sc, R, st, L, cur, stage, i, out); break;
                 case 1: shade_vertex_call<1>(sc, R, st, L, cur, stage, i, out); break;
@@ -841,12 +766,7 @@ __global__ void __launch_bounds__(128, TCPT_SHADE_MIN_BLOCKS) k_shade_all(const 
                 default: shade_vertex_call<8>(sc, R, st, L, cur, stage, i, out); break;
             }
         }
-        if (b < 6) {  // emissive hits and misses end the path: nothing to push (b is uniform over the block)
-            uint32_t pe, ps;
-            warp_push2(&st.counters[cur ^ 1], out.push_ext, &st.counters[sh], out.push_sh, &pe, &ps);
-            if (out.push_ext) { st.ext_o[cur ^ 1][pe] = out.eo; st.ext_d[cur ^ 1][pe] = out.ed; }
-            if (out.push_sh) { st.sh_o[ps] = out.so; st.sh_d[ps] = out.sd; st.sh_c[ps] = out.sc; }
-        }
+        push_rays(st, cur, sh, b, out);   // (b is uniform over the block)
     }
 }
 

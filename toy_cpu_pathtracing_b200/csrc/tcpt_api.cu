@@ -168,7 +168,7 @@ void srgb_xyz_to_rgb(float out[9]) {
 // device memory of one path slot: 14 float4 records (path state, both extension queues, hit record, shadow queue), the uint2 half of the
 // hit record and one order entry per shading bucket (ensure_state below allocates exactly this list)
 constexpr uint64_t kBytesPerSlot = 14 * sizeof(float4) + sizeof(uint2) + sizeof(tcpt::OrderEntry) * TCPT_N_BUCKETS;
-static_assert(kBytesPerSlot == (TCPT_ORDER_SLOT ? 304 : 268), "update the figure quoted in include/tcpt.h and DESIGN.md");
+static_assert(kBytesPerSlot == 304,"update the figure quoted in include/tcpt.h and DESIGN.md");
 
 int ensure_state(tcpt_ctx* ctx, uint32_t capacity) {
     if (ctx->st_capacity >= capacity) return TCPT_OK;
