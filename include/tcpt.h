@@ -184,6 +184,18 @@ int tcpt_render(tcpt_ctx* ctx, const tcpt_render_params* params, float* out_acc,
 int tcpt_render_device(tcpt_ctx* ctx, const tcpt_render_params* params, void* dev_acc, void* stream);
 /* Sensor::to_rgb on a device accumulator (after the NCCL reduce): dev_srgb = OETF(Reinhard(max(acc/spp,0))) */
 int tcpt_finalize_device(tcpt_ctx* ctx, const void* dev_acc, uint32_t width, uint32_t height, uint32_t spp, void* dev_srgb, void* stream);
+/* ---- adaptive sampling: the job `params` (spp = N) runs in rounds.  Round 0 renders samples [0, min_spp) of every pixel, every later
+ * round the next `step` samples (clipped at N) of the pixels still active.  After a round that ends at k < N an active pixel stops with
+ * count k when S1 and S2 are finite and e < threshold * (|m| + 1e-3), where, in f32 without contraction, y = (0.2126 r + 0.7152 g) +
+ * 0.0722 b of each sample's sensor RGB, S1 = sum y, S2 = sum y*y in sample order, m = S1/k, v = max(S2/k - m*m, 0), e = sqrt(v/(k - 1)).
+ * A pixel that never stops has count N.  A pixel with count k holds BITWISE the accumulator tcpt_render gives for the window [0, k) of the
+ * same job.  Outputs (host, any may be NULL, not all three): out_acc W*H*3 f32 sums, out_srgb W*H*3 f32 (tcpt_render's output transform
+ * with each pixel divided by its own count), out_spp W*H u32 counts.  Stats: paths = sum of the counts, render_ms = the whole call,
+ * passes / kernel_launches over all rounds.  Integrators pt / nee / mis, both samplers; max_slots is honoured; row_offset / row_stride
+ * and spp_begin / spp_end must be 0.  TCPT_ERR_INVALID: threshold negative or not finite, min_spp < 2 or > spp, step 0. */
+typedef struct { float threshold; uint32_t min_spp; uint32_t step; } tcpt_adaptive_params;
+int tcpt_render_adaptive(tcpt_ctx* ctx, const tcpt_render_params* params, const tcpt_adaptive_params* ap,
+                         float* out_acc, float* out_srgb, uint32_t* out_spp);
 int tcpt_get_stats(const tcpt_ctx* ctx, tcpt_stats* out);
 
 /* ---- multi-GPU (SURVEY.md 8b / 8e).  The reference has no distributed path; every (pixel, sample) is independent and the only shared

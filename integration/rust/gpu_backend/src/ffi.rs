@@ -112,6 +112,14 @@ pub struct TcptRenderParams {
     pub spp_end: u32,
     pub max_slots: u32,
 }
+/// Adaptive sampling (tcpt_render_adaptive): stop a pixel once the relative standard error of its mean luminance is below `threshold`
+#[repr(C)]
+#[derive(Clone, Copy, Default)]
+pub struct TcptAdaptiveParams {
+    pub threshold: f32,
+    pub min_spp: u32,
+    pub step: u32,
+}
 #[repr(C)]
 #[derive(Clone, Copy, Default)]
 pub struct TcptStats {
@@ -170,6 +178,8 @@ unsafe extern "C" {
     pub fn tcpt_render_device(ctx: *mut TcptCtx, params: *const TcptRenderParams, dev_acc: *mut c_void, stream: *mut c_void) -> c_int;
     pub fn tcpt_finalize_device(ctx: *mut TcptCtx, dev_acc: *const c_void, width: u32, height: u32, spp: u32, dev_srgb: *mut c_void,
                                 stream: *mut c_void) -> c_int;
+    pub fn tcpt_render_adaptive(ctx: *mut TcptCtx, params: *const TcptRenderParams, ap: *const TcptAdaptiveParams, out_acc: *mut f32,
+                                out_srgb: *mut f32, out_spp: *mut u32) -> c_int;
     pub fn tcpt_get_stats(ctx: *const TcptCtx, out: *mut TcptStats) -> c_int;
 
     // multi-GPU: one context per GPU; the library owns the NCCL communicator (include/tcpt.h "multi-GPU")

@@ -171,6 +171,23 @@ impl GpuRendererImage {
             panic!("tcpt_render: {}", last_error(self.ctx)); // the reference panics on errors too (main.rs:61,91,138,235)
         }
     }
+    /// Adaptive sampling (`tcpt_render_adaptive`): every pixel renders samples [0, min_spp), then `step` more per round until the
+    /// relative standard error of its mean luminance drops below `threshold` or it reaches the image's spp.  Each pixel's accumulator
+    /// is bitwise the one `render` gives for the window [0, count) of the same job; `pixels` are divided by each pixel's own count.
+    /// Returns the per-pixel sample counts (row major).
+    pub fn render_adaptive<S: GpuSampler>(&mut self, threshold: f32, min_spp: u32, step: u32) -> Vec<u32> {
+        self.params.sampler = S::ID;
+        let ap = TcptAdaptiveParams { threshold, min_spp, step };
+        let mut counts = vec![0u32; (self.params.width * self.params.height) as usize];
+        let rc = unsafe {
+            tcpt_render_adaptive(self.ctx, &self.params, &ap, self.accumulators.as_mut_ptr() as *mut f32, self.pixels.as_mut_ptr() as *mut f32,
+                                 counts.as_mut_ptr())
+        };
+        if rc != TCPT_OK {
+            panic!("tcpt_render_adaptive: {}", last_error(self.ctx));
+        }
+        counts
+    }
     /// One complete frame from every GPU of the communicator this context belongs to (`tcpt_comm_init`, one process per GPU): every
     /// rank calls it with the same image; rank 0's `pixels` / `accumulators` receive the frame after ONE ncclReduce inside the library.
     /// `TCPT_SHARD_TILE` reproduces the one-GPU film bit for bit, `TCPT_SHARD_SPP` balances best.

@@ -133,7 +133,9 @@ struct DRender {
     uint32_t log2_spp, n_base4_digits;  // ZSobolSampler::new (z_sobol_sampler.rs:179-196)
     // pass geometry: slot = s_local * n_pix + p_local ; owned pixel index = pix_begin + p_local ;
     // owned pixel k -> x = k % width, y = row_offset + (k / width) * row_stride ; sample_index = s_begin + s_local
+    // (with pix_list != nullptr the owned pixel index is pix_list[pix_begin + p_local] instead: a subset of the owned pixels, see owned_pixel)
     uint32_t n_pix, pix_begin, s_begin, s_count, row_offset, row_stride;
+    const uint32_t* pix_list;
     // exact division of a 32-bit number by n_pix / by width as one 64 x 64 -> high multiply: magic = floor(2^64 / d) + 1 (0 = divisor 1);
     // floor(n * magic / 2^64) == n / d for every n < 2^32 because n * (magic * d - 2^64) <= n * d < 2^64 (set by set_div_magics on the host)
     uint64_t n_pix_magic, width_magic;

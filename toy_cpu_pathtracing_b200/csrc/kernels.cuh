@@ -27,10 +27,16 @@ namespace tcpt {
 
 struct PathList { const uint32_t* xy; const uint32_t* sample; };  // explicit (pixel, sample) lists for tcpt_path_samples
 
+// owned pixel index of pass pixel p_local: consecutive from pix_begin, or the pix_begin + p_local-th entry of the pass's pixel list
+// (adaptive rounds: the frame indices of the pixels still active, in ascending order)
+__device__ __forceinline__ uint32_t owned_pixel(const DRender& R, uint32_t p_local) {
+    return R.pix_list ? __ldg(R.pix_list + R.pix_begin + p_local) : R.pix_begin + p_local;
+}
+
 __device__ __forceinline__ void path_coords(const DRender& R, const PathList& L, uint32_t slot, uint32_t* px, uint32_t* py, uint32_t* si) {
     if (L.xy) { *px = __ldg(L.xy + 2 * (size_t)slot); *py = __ldg(L.xy + 2 * (size_t)slot + 1); *si = __ldg(L.sample + slot); return; }
     const uint32_t s_local = div_magic(slot, R.n_pix_magic), p_local = slot - s_local * R.n_pix;
-    const uint32_t k = R.pix_begin + p_local;
+    const uint32_t k = owned_pixel(R, p_local);
     const uint32_t row = div_magic(k, R.width_magic);
     *px = k - row * R.width;
     *py = R.row_offset + row * R.row_stride;
@@ -75,7 +81,7 @@ __global__ void __launch_bounds__(256) k_sobol_pass(uint32_t* __restrict__ table
     const size_t total = (size_t)R.n_pix * dims;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
         const uint32_t dim = (uint32_t)(i / R.n_pix), p_local = (uint32_t)(i - (size_t)dim * R.n_pix);
-        const uint32_t k = R.pix_begin + p_local, row = k / R.width;
+        const uint32_t k = owned_pixel(R, p_local), row = k / R.width;
         const uint32_t px = k - row * R.width, py = R.row_offset + row * R.row_stride;
         table[(size_t)(R.prefix_dims + dim) * R.prefix_stride + (size_t)py * R.width + px] =
             DSampler::pass_entry(DSampler::morton_of(px, py, R.s_begin, R.log2_spp), dim, R.log2_spp, iv);
@@ -93,7 +99,7 @@ __global__ void __launch_bounds__(256) k_sobol_pass_cached(uint32_t* __restrict_
     const uint32_t tag_new = (R.s_begin >> (2u * iv)) & ((1u << (2u * levels)) - 1u);
     // one thread per PIXEL, looping over the dimensions: coordinates and Morton code once per pixel; a warp's accesses to a row stay contiguous
     for (uint32_t p_local = blockIdx.x * blockDim.x + threadIdx.x; p_local < R.n_pix; p_local += gridDim.x * blockDim.x) {
-        const uint32_t k = R.pix_begin + p_local, row = div_magic(k, R.width_magic);
+        const uint32_t k = owned_pixel(R, p_local), row = div_magic(k, R.width_magic);
         const uint32_t px = k - row * R.width, py = R.row_offset + row * R.row_stride;
         const size_t col = (size_t)py * R.width + px;
         const uint32_t morton = DSampler::morton_of(px, py, R.s_begin, R.log2_spp);
@@ -179,7 +185,7 @@ __global__ void __launch_bounds__(256) k_generate_pixels(const __grid_constant__
     const uint32_t d_uv = with_lambda ? 1u : 0u;
     const uint64_t h_u = DSampler::hash_of(1u, f), h_uv = DSampler::hash_of(d_uv + 2u, f);
     for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < R.n_pix; p += stride) {
-        const uint32_t k = R.pix_begin + p;
+        const uint32_t k = owned_pixel(R, p);
         const uint32_t row = div_magic(k, R.width_magic);
         const uint32_t px = k - row * R.width, py = R.row_offset + row * R.row_stride;
         const uint32_t pix = py * R.width + px;
@@ -811,7 +817,7 @@ __global__ void __launch_bounds__(128) k_aov(const __grid_constant__ DScene sc, 
 __global__ void __launch_bounds__(256) k_film(const __grid_constant__ DRender R, const float4* __restrict__ rgb, float* __restrict__ acc) {
     const uint32_t stride = gridDim.x * blockDim.x;
     for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < R.n_pix; p += stride) {
-        const uint32_t k = R.pix_begin + p;
+        const uint32_t k = R.pix_begin + p;   // passes over a pixel list (R.pix_list) use k_film_moments
         const uint32_t row = k / R.width;
         const uint32_t px = k - row * R.width, py = R.row_offset + row * R.row_stride;
         float* a = acc + 3 * ((size_t)py * R.width + px);
@@ -835,6 +841,141 @@ __global__ void __launch_bounds__(256) k_finalize(const float* __restrict__ acc,
         if (mode == 0) c = c / (1.0f + c);
         out[i] = linear_to_srgb(c);
     }
+}
+
+// ---------------------------------------------------------------- adaptive sampling (tcpt_render_adaptive)
+// k_film plus the per-pixel luminance moments of the stopping rule: mom[pixel] = {S1, S2} += {y, y*y} with y = (0.2126 r + 0.7152 g) + 0.0722 b
+// of every sample the film adds, in the same loop and the same order (f32, no contraction: the library builds with --fmad=false)
+__global__ void __launch_bounds__(256) k_film_moments(const __grid_constant__ DRender R, const float4* __restrict__ rgb, float* __restrict__ acc, float2* __restrict__ mom) {
+    const uint32_t stride = gridDim.x * blockDim.x;
+    for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < R.n_pix; p += stride) {
+        const uint32_t k = owned_pixel(R, p);
+        const uint32_t row = k / R.width;
+        const uint32_t px = k - row * R.width, py = R.row_offset + row * R.row_stride;
+        const size_t pix = (size_t)py * R.width + px;
+        float* a = acc + 3 * pix;
+        float r = a[0], g = a[1], b = a[2];
+        float2 m = mom[pix];
+        for (uint32_t s = 0; s < R.s_count; ++s) {
+            const float4 v = rgb[(size_t)s * R.n_pix + p];
+            r += v.x; g += v.y; b += v.z;
+            const float y = (0.2126f * v.x + 0.7152f * v.y) + 0.0722f * v.z;
+            m.x += y; m.y += y * y;
+        }
+        a[0] = r; a[1] = g; a[2] = b;
+        mom[pix] = m;
+    }
+}
+
+// the stopping rule after k samples: relative standard error of the mean luminance below `threshold`, with an absolute floor of 1e-3
+// (IEEE division and square root; a pixel whose sums are not finite never stops)
+__device__ __forceinline__ bool adaptive_converged(float2 m2, uint32_t k, float threshold) {
+    const float kf = (float)k;
+    const float m = m2.x / kf;
+    float v = m2.y / kf - m * m;
+    v = v > 0.0f ? v : 0.0f;
+    const float e = sqrtf(v / (kf - 1.0f));
+    return isfinite(m2.x) && isfinite(m2.y) && e < threshold * (fabsf(m) + 1e-3f);
+}
+
+// Stream compaction of the active pixel list, count / scan / scatter: tiles of TCPT_SELECT_THREADS x TCPT_SELECT_ITEMS consecutive entries,
+// each thread owning TCPT_SELECT_ITEMS consecutive ones, so the survivors keep their (ascending) order.  Deterministic: no atomics.
+#define TCPT_SELECT_THREADS 256
+#define TCPT_SELECT_ITEMS 4
+#define TCPT_SELECT_TILE (TCPT_SELECT_THREADS * TCPT_SELECT_ITEMS)
+
+// exclusive prefix sum of v over the block (blockDim.x a multiple of 32, at most 1024); *total = the block's sum.  Every thread must call it.
+__device__ __forceinline__ uint32_t block_exclusive_scan(uint32_t v, uint32_t* total) {
+    __shared__ uint32_t warp_sums[32];
+    const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5, n_warps = blockDim.x >> 5;
+    uint32_t x = v;
+#pragma unroll
+    for (uint32_t o = 1; o < 32u; o <<= 1) { const uint32_t y = __shfl_up_sync(0xffffffffu, x, o); if (lane >= o) x += y; }
+    if (lane == 31u) warp_sums[warp] = x;
+    __syncthreads();
+    if (warp == 0) {
+        uint32_t w = lane < n_warps ? warp_sums[lane] : 0u;
+#pragma unroll
+        for (uint32_t o = 1; o < 32u; o <<= 1) { const uint32_t y = __shfl_up_sync(0xffffffffu, w, o); if (lane >= o) w += y; }
+        if (lane < n_warps) warp_sums[lane] = w;
+    }
+    __syncthreads();
+    const uint32_t excl = x - v + (warp ? warp_sums[warp - 1] : 0u);
+    *total = warp_sums[n_warps - 1];
+    __syncthreads();   // warp_sums is reused by the next call
+    return excl;
+}
+
+// this thread's entries of the active list (nullptr = the identity list 0 .. n - 1): frame pixel indices and the mask of the ones that stay active
+__device__ __forceinline__ uint32_t adaptive_items(const uint32_t* __restrict__ list, uint32_t n, const float2* __restrict__ mom, uint32_t k, float threshold,
+                                                   uint32_t pix[TCPT_SELECT_ITEMS], uint32_t* valid) {
+    const uint32_t first = (blockIdx.x * TCPT_SELECT_THREADS + threadIdx.x) * TCPT_SELECT_ITEMS;
+    uint32_t keep = 0u, ok = 0u;
+#pragma unroll
+    for (uint32_t j = 0; j < TCPT_SELECT_ITEMS; ++j) {
+        const uint32_t i = first + j;
+        pix[j] = 0u;
+        if (i >= n) continue;
+        pix[j] = list ? list[i] : i;
+        ok |= 1u << j;
+        if (!adaptive_converged(mom[pix[j]], k, threshold)) keep |= 1u << j;
+    }
+    *valid = ok;
+    return keep;
+}
+
+// count: every pixel that stops gets its sample count k; tile_counts[tile] = survivors of the tile
+__global__ void __launch_bounds__(TCPT_SELECT_THREADS) k_adaptive_count(const uint32_t* __restrict__ list, uint32_t n, const float2* __restrict__ mom,
+                                                                        uint32_t k, float threshold, uint32_t* __restrict__ counts, uint32_t* __restrict__ tile_counts) {
+    uint32_t pix[TCPT_SELECT_ITEMS], valid;
+    const uint32_t keep = adaptive_items(list, n, mom, k, threshold, pix, &valid);
+#pragma unroll
+    for (uint32_t j = 0; j < TCPT_SELECT_ITEMS; ++j)
+        if (((valid & ~keep) >> j) & 1u) counts[pix[j]] = k;
+    uint32_t total;
+    block_exclusive_scan((uint32_t)__popc(keep), &total);
+    if (threadIdx.x == 0) tile_counts[blockIdx.x] = total;
+}
+
+// scan: tile_counts -> exclusive offsets in place, *n_out = number of survivors (one block of 1024 threads walks the tiles in order)
+__global__ void __launch_bounds__(1024) k_adaptive_scan(uint32_t* __restrict__ tile_counts, uint32_t n_tiles, uint32_t* __restrict__ n_out) {
+    uint32_t carry = 0u;
+    for (uint32_t base = 0; base < n_tiles; base += blockDim.x) {
+        const uint32_t i = base + threadIdx.x;
+        const uint32_t v = i < n_tiles ? tile_counts[i] : 0u;
+        uint32_t sum;
+        const uint32_t e = block_exclusive_scan(v, &sum);
+        if (i < n_tiles) tile_counts[i] = carry + e;
+        carry += sum;
+    }
+    if (threadIdx.x == 0) *n_out = carry;
+}
+
+// scatter: the survivors of every tile to list_out from the tile's offset, in list order (the rule is evaluated again: same inputs, same answer)
+__global__ void __launch_bounds__(TCPT_SELECT_THREADS) k_adaptive_scatter(const uint32_t* __restrict__ list, uint32_t n, const float2* __restrict__ mom,
+                                                                          uint32_t k, float threshold, const uint32_t* __restrict__ tile_offsets, uint32_t* __restrict__ list_out) {
+    uint32_t pix[TCPT_SELECT_ITEMS], valid;
+    const uint32_t keep = adaptive_items(list, n, mom, k, threshold, pix, &valid);
+    uint32_t total;
+    uint32_t o = tile_offsets[blockIdx.x] + block_exclusive_scan((uint32_t)__popc(keep), &total);
+#pragma unroll
+    for (uint32_t j = 0; j < TCPT_SELECT_ITEMS; ++j)
+        if ((keep >> j) & 1u) list_out[o++] = pix[j];
+}
+
+// k_finalize mode 0 with a per-pixel divisor: the value of a pixel with count k is bitwise what k_finalize gives with spp = k
+__global__ void __launch_bounds__(256) k_finalize_counts(const float* __restrict__ acc, const uint32_t* __restrict__ counts, float* __restrict__ out, uint32_t n_values) {
+    const uint32_t stride = gridDim.x * blockDim.x;
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_values; i += stride) {
+        float c = acc[i] / (float)counts[i / 3u];
+        c = c > 0.0f ? c : 0.0f;
+        c = c / (1.0f + c);
+        out[i] = linear_to_srgb(c);
+    }
+}
+
+__global__ void __launch_bounds__(256) k_fill_u32(uint32_t* __restrict__ p, uint32_t n, uint32_t value) {
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) p[i] = value;
 }
 
 // ---------------------------------------------------------------- single-stage probes for parity tests and the traversal micro-benchmark

@@ -97,7 +97,9 @@ struct tcpt_ctx {
     std::vector<cudaEvent_t> ev_pool; size_t ev_used = 0; std::vector<int> ev_stage;  // stage timing (see StageTimer)
     // tcpt_render's own film buffers (grow-only) and the caller's output buffers currently page-locked for direct DMA
     float* film_acc = nullptr; float* film_srgb = nullptr; size_t film_cap = 0;
-    HostPin pins[2];
+    HostPin pins[3];   // out_acc, out_srgb, out_spp
+    // tcpt_render_adaptive's buffers (grow-only, in pixels): luminance moments (float2), sample counts, two active lists, compaction scratch
+    void* adapt_buf = nullptr; size_t adapt_cap = 0;
     // ZSobol pixel-prefix table (DSampler::sample_index), cached per (width, height, log2_spp); grows when more dimensions are asked for
     float half_lin = 0.0f; int32_t half_zi = -1;   // DScene::half_lin / half_zi (tcpt_set_tables)
     void* trace_scratch = nullptr; size_t trace_scratch_cap = 0;   // device staging of tcpt_trace (rays in, hit records out), kept between calls
@@ -369,8 +371,8 @@ static void debug_dump(tcpt_ctx* ctx, const char* what, uint32_t stage, int cur,
                  so.x, so.y, so.z, sd.x, sd.y, sd.z, so.w, sc_.x, sc_.y, sc_.z, sc_.w);
 }
 
-// one pass = generate + (max_depth + 1) x {closest, shade, shadow} (+ film when acc != nullptr)
-int run_pass(tcpt_ctx* ctx, const DRender& R, const DCamera& cam, const PathList& L, uint32_t n_slots, float* dev_acc, cudaStream_t stream) {
+// one pass = generate + (max_depth + 1) x {closest, shade, shadow} (+ film when acc != nullptr; with the luminance moments when dev_mom != nullptr)
+int run_pass(tcpt_ctx* ctx, const DRender& R, const DCamera& cam, const PathList& L, uint32_t n_slots, float* dev_acc, cudaStream_t stream, float2* dev_mom = nullptr) {
     const DScene& sc = ctx->dev.view;
     const DState& st = ctx->st;
     const bool count = ctx->opt.count_tests != 0;
@@ -458,7 +460,8 @@ int run_pass(tcpt_ctx* ctx, const DRender& R, const DCamera& cam, const PathList
     }
     if (dev_acc) {
         StageTimer t(ctx, STAGE_FILM, stream);
-        k_film<<<grid_for(ctx, R.n_pix, 256), 256, 0, stream>>>(R, st.rgb, dev_acc);
+        if (dev_mom) k_film_moments<<<grid_for(ctx, R.n_pix, 256), 256, 0, stream>>>(R, st.rgb, dev_acc, dev_mom);
+        else k_film<<<grid_for(ctx, R.n_pix, 256), 256, 0, stream>>>(R, st.rgb, dev_acc);
         ctx->stats.kernel_launches++;
     }
     ctx->stats.passes++;
@@ -480,23 +483,17 @@ void reset_stats(tcpt_ctx* ctx) {
     ctx->ev_used = 0; ctx->ev_stage.clear();
 }
 
-int render_into(tcpt_ctx* ctx, const tcpt_render_params* p, float* dev_acc, cudaStream_t stream) {
-    DRender R; DCamera cam;
-    int rc = make_render(ctx, p, R, cam);
-    if (rc) return rc;
-    if (R.row_offset >= R.row_stride) return fail(ctx, TCPT_ERR_INVALID, "render: row_offset must be < row_stride");
-    rc = ensure_sobol_prefix(ctx, R, stream);
-    if (rc) return rc;
-    const uint32_t s0 = (p->spp_begin == 0 && p->spp_end == 0) ? 0 : p->spp_begin;
-    const uint32_t s1 = (p->spp_begin == 0 && p->spp_end == 0) ? p->spp : p->spp_end;
-    if (s1 > p->spp || s0 > s1) return fail(ctx, TCPT_ERR_INVALID, "render: bad sample range");
-    const uint32_t rows = R.row_offset < p->height ? (p->height - R.row_offset + R.row_stride - 1) / R.row_stride : 0;
-    const uint64_t owned = (uint64_t)rows * p->width;
-    if (owned == 0 || s0 == s1) return TCPT_OK;
+// The pass loop of a job: `owned` pixels -- owned indices 0 .. owned - 1, or the entries of the device list `pix_list` (frame indices of a
+// job with row_offset 0 / row_stride 1) -- times the sample window [s0, s1), cut into (pixel block x sample window) passes that fit the
+// path-slot budget.  R comes from make_render + ensure_sobol_prefix.  dev_mom != nullptr: the film also adds the luminance moments.
+int render_passes(tcpt_ctx* ctx, const DRender& R, const DCamera& cam, uint64_t owned, const uint32_t* pix_list, uint32_t s0, uint32_t s1,
+                  uint32_t max_slots, float* dev_acc, float2* dev_mom, cudaStream_t stream) {
+    if (pix_list && dev_acc && !dev_mom) return fail(ctx, TCPT_ERR_INVALID, "render: a pass over a pixel list films through k_film_moments");
+    int rc = TCPT_OK;
     // Path-slot budget of one pass.  Every pass pays a fixed latency (about 35 launches whose deep-bounce queues are nearly
     // empty: 4 to 8 ms on the 4K frame), so passes are made as large as memory comfortably allows: up to 128 Mi slots
     // (304 B each: 40 GB of the 180 GB), never more than 45 % of the memory that is free.
-    uint64_t budget = p->max_slots;
+    uint64_t budget = max_slots;
     if (budget == 0) {
         if (ctx->default_slots == 0) {  // asked once per context: cudaMemGetInfo was measured to stall a render by up to 80 ms
             size_t free_b = 0, total_b = 0;
@@ -518,7 +515,7 @@ int render_into(tcpt_ctx* ctx, const tcpt_render_params* p, float* dev_acc, cuda
         if (sc_per_pass > s1 - s0) sc_per_pass = s1 - s0;
         rc = ensure_state(ctx, (uint32_t)((uint64_t)np * sc_per_pass));
         // the budget is a guess made once per context (other tenants, a Z-Sobol table that has grown since): shrink the pass instead of failing
-        if (rc == TCPT_ERR_NOMEM && p->max_slots == 0 && budget > (1ull << 20)) { budget >>= 1; ctx->default_slots = budget; continue; }
+        if (rc == TCPT_ERR_NOMEM && max_slots == 0 && budget > (1ull << 20)) { budget >>= 1; ctx->default_slots = budget; continue; }
         break;
     }
     if (rc) return rc;
@@ -527,14 +524,30 @@ int render_into(tcpt_ctx* ctx, const tcpt_render_params* p, float* dev_acc, cuda
         const uint32_t n_pix = (uint32_t)((owned - pb) < np ? (owned - pb) : np);
         for (uint32_t sb = s0; sb < s1; sb += sc_per_pass) {
             DRender Rp = R;
-            Rp.n_pix = n_pix; Rp.pix_begin = (uint32_t)pb; Rp.s_begin = sb; Rp.s_count = (s1 - sb) < sc_per_pass ? (s1 - sb) : sc_per_pass;
+            Rp.n_pix = n_pix; Rp.pix_begin = (uint32_t)pb; Rp.pix_list = pix_list; Rp.s_begin = sb; Rp.s_count = (s1 - sb) < sc_per_pass ? (s1 - sb) : sc_per_pass;
             set_div_magics(Rp);
             build_sobol_pass(ctx, Rp, stream);
-            rc = run_pass(ctx, Rp, cam, none, n_pix * Rp.s_count, dev_acc, stream);
+            rc = run_pass(ctx, Rp, cam, none, n_pix * Rp.s_count, dev_acc, stream, dev_mom);
             if (rc) return rc;
         }
     }
     return TCPT_OK;
+}
+
+int render_into(tcpt_ctx* ctx, const tcpt_render_params* p, float* dev_acc, cudaStream_t stream) {
+    DRender R; DCamera cam;
+    int rc = make_render(ctx, p, R, cam);
+    if (rc) return rc;
+    if (R.row_offset >= R.row_stride) return fail(ctx, TCPT_ERR_INVALID, "render: row_offset must be < row_stride");
+    rc = ensure_sobol_prefix(ctx, R, stream);
+    if (rc) return rc;
+    const uint32_t s0 = (p->spp_begin == 0 && p->spp_end == 0) ? 0 : p->spp_begin;
+    const uint32_t s1 = (p->spp_begin == 0 && p->spp_end == 0) ? p->spp : p->spp_end;
+    if (s1 > p->spp || s0 > s1) return fail(ctx, TCPT_ERR_INVALID, "render: bad sample range");
+    const uint32_t rows = R.row_offset < p->height ? (p->height - R.row_offset + R.row_stride - 1) / R.row_stride : 0;
+    const uint64_t owned = (uint64_t)rows * p->width;
+    if (owned == 0 || s0 == s1) return TCPT_OK;
+    return render_passes(ctx, R, cam, owned, nullptr, s0, s1, p->max_slots, dev_acc, nullptr, stream);
 }
 
 void unpin_all(tcpt_ctx* ctx) {
@@ -543,7 +556,7 @@ void unpin_all(tcpt_ctx* ctx) {
 
 // Device -> caller's host buffer.  With option "pin_host_buffers" the buffer is page-locked once (and stays so while the same
 // pointer is passed again) so the copy is a direct DMA at PCIe rate instead of a staged pageable copy.
-int copy_out(tcpt_ctx* ctx, int slot, float* host, const float* dev, size_t bytes) {
+int copy_out(tcpt_ctx* ctx, int slot, void* host, const void* dev, size_t bytes) {
     if (ctx->opt.pin_host_buffers) {
         HostPin& h = ctx->pins[slot];
         if (h.ptr != host || h.bytes != bytes) {
@@ -555,6 +568,37 @@ int copy_out(tcpt_ctx* ctx, int slot, float* host, const float* dev, size_t byte
     }
     CU(cudaMemcpyAsync(host, dev, bytes, cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
+    return TCPT_OK;
+}
+
+// the context's film buffers (tcpt_render and tcpt_render_adaptive), grown to n floats each
+int ensure_film(tcpt_ctx* ctx, size_t n) {
+    if (ctx->film_cap >= n) return TCPT_OK;
+    if (ctx->film_acc) cudaFree(ctx->film_acc);
+    if (ctx->film_srgb) cudaFree(ctx->film_srgb);
+    ctx->film_acc = ctx->film_srgb = nullptr; ctx->film_cap = 0;
+    CU(cudaMalloc((void**)&ctx->film_acc, n * sizeof(float)));
+    CU(cudaMalloc((void**)&ctx->film_srgb, n * sizeof(float)));
+    ctx->film_cap = n;
+    return TCPT_OK;
+}
+
+// tcpt_render_adaptive's per-pixel buffers, carved from one grow-only allocation
+struct AdaptiveBuffers { float2* mom; uint32_t* counts; uint32_t* list[2]; uint32_t* tiles; uint32_t* n_active; };
+size_t adaptive_bytes(size_t n_pix) { return n_pix * (sizeof(float2) + 3 * sizeof(uint32_t)) + ((n_pix + TCPT_SELECT_TILE - 1) / TCPT_SELECT_TILE + 1) * sizeof(uint32_t); }
+int ensure_adaptive(tcpt_ctx* ctx, size_t n_pix, AdaptiveBuffers& b) {
+    if (ctx->adapt_cap < n_pix) {
+        if (ctx->adapt_buf) { cudaStreamSynchronize(ctx->stream); cudaFree(ctx->adapt_buf); }
+        ctx->adapt_buf = nullptr; ctx->adapt_cap = 0;
+        CU(cudaMalloc(&ctx->adapt_buf, adaptive_bytes(n_pix)));
+        ctx->adapt_cap = n_pix;
+    }
+    const size_t cap = ctx->adapt_cap;
+    b.mom = (float2*)ctx->adapt_buf;
+    b.counts = (uint32_t*)(b.mom + cap);
+    b.list[0] = b.counts + cap; b.list[1] = b.list[0] + cap;
+    b.n_active = b.list[1] + cap;
+    b.tiles = b.n_active + 1;
     return TCPT_OK;
 }
 
@@ -599,6 +643,7 @@ void tcpt_destroy(tcpt_ctx* ctx) {
     unpin_all(ctx);
     if (ctx->film_acc) cudaFree(ctx->film_acc);
     if (ctx->film_srgb) cudaFree(ctx->film_srgb);
+    if (ctx->adapt_buf) cudaFree(ctx->adapt_buf);
     if (ctx->d_cmf) cudaFree(ctx->d_cmf);
     if (ctx->d_sobol_bytes) cudaFree(ctx->d_sobol_bytes);
     if (ctx->d_presets) cudaFree(ctx->d_presets);
@@ -1073,16 +1118,10 @@ int tcpt_render(tcpt_ctx* ctx, const tcpt_render_params* params, float* out_acc,
     if (!ctx->stream) return fail(ctx, TCPT_ERR_CUDA, "no CUDA device");
     CU(cudaSetDevice(ctx->device));
     const size_t n = (size_t)params->width * params->height * 3;
-    if (ctx->film_cap < n) {
-        if (ctx->film_acc) cudaFree(ctx->film_acc);
-        if (ctx->film_srgb) cudaFree(ctx->film_srgb);
-        ctx->film_acc = ctx->film_srgb = nullptr; ctx->film_cap = 0;
-        CU(cudaMalloc((void**)&ctx->film_acc, n * sizeof(float)));
-        CU(cudaMalloc((void**)&ctx->film_srgb, n * sizeof(float)));
-        ctx->film_cap = n;
-    }
+    int rc = ensure_film(ctx, n);
+    if (rc) return rc;
     CU(cudaMemsetAsync(ctx->film_acc, 0, n * sizeof(float), ctx->stream));
-    int rc = tcpt_render_device(ctx, params, ctx->film_acc, nullptr);
+    rc = tcpt_render_device(ctx, params, ctx->film_acc, nullptr);
     if (rc) return rc;
     if (out_acc && (rc = copy_out(ctx, 0, out_acc, ctx->film_acc, n * sizeof(float))) != TCPT_OK) return rc;
     if (out_srgb) {
@@ -1094,6 +1133,71 @@ int tcpt_render(tcpt_ctx* ctx, const tcpt_render_params* params, float* out_acc,
     return TCPT_OK;
 }
 
+// Adaptive sampling (include/tcpt.h): rounds of render_passes over the pixels still active.  Round 0 takes every pixel (no list); after
+// each round that ends below spp, k_adaptive_count / _scan / _scatter write the counts of the pixels that stop and compact the others,
+// in ascending pixel order, into the next list.  One 4-byte device -> host copy per round (the active count) sizes the next round.
+int tcpt_render_adaptive(tcpt_ctx* ctx, const tcpt_render_params* params, const tcpt_adaptive_params* ap, float* out_acc, float* out_srgb, uint32_t* out_spp) {
+    if (!ctx || !params || !ap) return TCPT_ERR_INVALID;
+    if (!out_acc && !out_srgb && !out_spp) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive: no output buffer");
+    if (!std::isfinite(ap->threshold) || ap->threshold < 0.0f) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive: threshold must be finite and >= 0");
+    if (ap->min_spp < 2 || ap->min_spp > params->spp) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive: min_spp must lie in [2, spp]");
+    if (ap->step == 0) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive: step must be positive");
+    if (params->integrator < TCPT_INTEGRATOR_PT || params->integrator > TCPT_INTEGRATOR_MIS) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive: integrators pt, nee and mis only");
+    if (params->row_offset || params->row_stride) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive: row_offset / row_stride must be 0 (whole frame)");
+    if (params->spp_begin || params->spp_end) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive: spp_begin / spp_end must be 0 (all samples)");
+    if (!ctx->stream) return fail(ctx, TCPT_ERR_CUDA, "no CUDA device");
+    CU(cudaSetDevice(ctx->device));
+    DRender R; DCamera cam;
+    int rc = make_render(ctx, params, R, cam);
+    if (rc) return rc;
+    const uint64_t n_pix64 = (uint64_t)params->width * params->height;
+    if (n_pix64 * 3 > 0xffffffffull) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive: frame too large");
+    const uint32_t n_pix = (uint32_t)n_pix64, N = params->spp;
+    const size_t n = (size_t)n_pix * 3;
+    cudaStream_t s = ctx->stream;
+    AdaptiveBuffers B;
+    if ((rc = ensure_film(ctx, n)) != TCPT_OK || (rc = ensure_adaptive(ctx, n_pix, B)) != TCPT_OK) return rc;
+    reset_stats(ctx);
+    CU(cudaEventRecord(ctx->ev0, s));
+    if ((rc = ensure_sobol_prefix(ctx, R, s)) != TCPT_OK) return rc;
+    CU(cudaMemsetAsync(ctx->film_acc, 0, n * sizeof(float), s));
+    CU(cudaMemsetAsync(B.mom, 0, (size_t)n_pix * sizeof(float2), s));
+    k_fill_u32<<<grid_for(ctx, n_pix, 256), 256, 0, s>>>(B.counts, n_pix, N);   // a pixel that never stops has count N
+    ctx->stats.kernel_launches++;
+    uint32_t k = 0, active = n_pix, cur = 0;
+    const uint32_t* list = nullptr;   // round 0: every pixel, in order
+    while (active > 0) {
+        const uint64_t want = k == 0 ? ap->min_spp : (uint64_t)k + ap->step;
+        const uint32_t k_next = want < N ? (uint32_t)want : N;
+        if ((rc = render_passes(ctx, R, cam, active, list, k, k_next, params->max_slots, ctx->film_acc, B.mom, s)) != TCPT_OK) return rc;
+        k = k_next;
+        if (k >= N) break;
+        const uint32_t n_tiles = (active + TCPT_SELECT_TILE - 1) / TCPT_SELECT_TILE;
+        k_adaptive_count<<<n_tiles, TCPT_SELECT_THREADS, 0, s>>>(list, active, B.mom, k, ap->threshold, B.counts, B.tiles);
+        k_adaptive_scan<<<1, 1024, 0, s>>>(B.tiles, n_tiles, B.n_active);
+        k_adaptive_scatter<<<n_tiles, TCPT_SELECT_THREADS, 0, s>>>(list, active, B.mom, k, ap->threshold, B.tiles, B.list[cur]);
+        ctx->stats.kernel_launches += 3;
+        CU(cudaGetLastError());
+        CU(cudaMemcpyAsync(&active, B.n_active, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+        CU(cudaStreamSynchronize(s));
+        list = B.list[cur]; cur ^= 1u;
+    }
+    if (out_srgb) {
+        k_finalize_counts<<<grid_for(ctx, n, 256), 256, 0, s>>>(ctx->film_acc, B.counts, ctx->film_srgb, (uint32_t)n);
+        ctx->stats.kernel_launches++;
+        CU(cudaGetLastError());
+    }
+    CU(cudaEventRecord(ctx->ev1, s));
+    CU(cudaEventSynchronize(ctx->ev1));
+    float ms = 0; CU(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+    ctx->stats.render_ms = ms;
+    collect_stage_times(ctx);
+    if ((rc = fetch_stats(ctx)) != TCPT_OK) return rc;
+    if (out_acc && (rc = copy_out(ctx, 0, out_acc, ctx->film_acc, n * sizeof(float))) != TCPT_OK) return rc;
+    if (out_srgb && (rc = copy_out(ctx, 1, out_srgb, ctx->film_srgb, n * sizeof(float))) != TCPT_OK) return rc;
+    if (out_spp && (rc = copy_out(ctx, 2, out_spp, B.counts, (size_t)n_pix * sizeof(uint32_t))) != TCPT_OK) return rc;
+    return TCPT_OK;
+}
 
 // ---------------------------------------------------------------- multi-GPU: NCCL inside the library (SURVEY.md 8b / 8e)
 int tcpt_comm_get_unique_id(void* id128) {

@@ -116,6 +116,7 @@ class RendererImage:                  # renderer/src/renderer.rs:101-149
         self.width, self.height, self.renderer = int(width), int(height), renderer
         self.pixels = np.zeros((self.height, self.width, 3), dtype=f32)       # tone-mapped sRGB, what `pixels` holds in the reference
         self.accumulators = np.zeros((self.height, self.width, 3), dtype=f32)  # Sensor accumulators (linear sRGB sums)
+        self.sample_counts = np.zeros((self.height, self.width), dtype=np.uint32)  # samples per pixel of the last render_adaptive
         self.stats: dict = {}
 
     @classmethod
@@ -134,6 +135,28 @@ class RendererImage:                  # renderer/src/renderer.rs:101-149
         ctx.check(ctx.lib.tcpt_render(ctx.handle, C.byref(p), capi.as_ptr(self.accumulators, C.c_float) if want_accumulators else None,
                                       capi.as_ptr(self.pixels, C.c_float)))
         self.stats = ctx.stats()
+        return self
+
+    def render_adaptive(self, sampler=ZSobolSampler, threshold: float = 0.01, min_spp: int = 64, step: int = 64,
+                        want_accumulators: bool = True, max_slots: int = 0) -> "RendererImage":
+        """Adaptive sampling (tcpt_render_adaptive): every pixel renders samples [0, min_spp), then `step` more per round while the
+        relative standard error of its mean luminance is at least `threshold` (absolute floor 1e-3), up to the renderer's spp.
+        `sample_counts` receives each pixel's count k; its accumulator is bitwise what `render` gives for the sample window [0, k) of the
+        same job, and `pixels` holds the output transform of accumulator / k.  stats["rounds"] = rounds the job took."""
+        r = self.renderer
+        ctx = r.args.scene.ctx
+        if not r.args.scene.built:
+            r.args.scene.build(r.args.camera)
+        p = r.params(sampler, max_slots=max_slots)
+        ap = capi.AdaptiveParams(float(threshold), int(min_spp), int(step))
+        ctx.set_option("pin_host_buffers", 1)
+        self._pinned_ctx = ctx
+        ctx.check(ctx.lib.tcpt_render_adaptive(ctx.handle, C.byref(p), C.byref(ap),
+                                               capi.as_ptr(self.accumulators, C.c_float) if want_accumulators else None,
+                                               capi.as_ptr(self.pixels, C.c_float), capi.as_ptr(self.sample_counts, C.c_uint32)))
+        self.stats = ctx.stats()
+        # the last round ends at the largest count: round 0 reaches min_spp, every later one `step` more (the last clipped at spp)
+        self.stats["rounds"] = 1 + -(-(int(self.sample_counts.max()) - int(min_spp)) // int(step))
         return self
 
     def render_sharded(self, sampler=ZSobolSampler, mode: str = "tile", want_accumulators: bool = True, spp_window=None, max_slots: int = 0) -> "RendererImage":
