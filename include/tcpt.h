@@ -192,10 +192,21 @@ int tcpt_finalize_device(tcpt_ctx* ctx, const void* dev_acc, uint32_t width, uin
  * same job.  Outputs (host, any may be NULL, not all three): out_acc W*H*3 f32 sums, out_srgb W*H*3 f32 (tcpt_render's output transform
  * with each pixel divided by its own count), out_spp W*H u32 counts.  Stats: paths = sum of the counts, render_ms = the whole call,
  * passes / kernel_launches over all rounds.  Integrators pt / nee / mis, both samplers; max_slots is honoured; row_offset / row_stride
- * and spp_begin / spp_end must be 0.  TCPT_ERR_INVALID: threshold negative or not finite, min_spp < 2 or > spp, step 0. */
+ * and spp_begin / spp_end must be 0.  TCPT_ERR_INVALID: threshold negative or not finite, min_spp < 2 or > spp, step 0.  A communicator on
+ * the context (tcpt_comm_init, a tcpt_group context) is not used: the whole frame is rendered and returned by this GPU alone, on any rank
+ * (tcpt_render_adaptive_sharded is the multi-GPU form). */
 typedef struct { float threshold; uint32_t min_spp; uint32_t step; } tcpt_adaptive_params;
 int tcpt_render_adaptive(tcpt_ctx* ctx, const tcpt_render_params* params, const tcpt_adaptive_params* ap,
                          float* out_acc, float* out_srgb, uint32_t* out_spp);
+/* One row shard of an adaptive job into caller-owned DEVICE buffers on `stream` (cudaStream_t or NULL, as in tcpt_render_device); no
+ * collective.  `params` may carry a row shard, any row_offset < row_stride as tcpt_shard_params(..., TCPT_SHARD_TILE, ...) makes it;
+ * spp_begin / spp_end must be 0 (tcpt_shard_params writes the job's range [0, spp) there: reset both).  The rounds, the rule and the checks on `ap` and the integrator are those of tcpt_render_adaptive, over
+ * the owned pixels only: each owned pixel stops exactly where it stops in tcpt_render_adaptive of the whole job.  dev_acc (W*H*3 f32) and
+ * dev_spp (W*H u32) are both required: each owned pixel's sum is ADDED into dev_acc (the caller zeroes it) and its count WRITTEN into
+ * dev_spp; no other pixel of either buffer is touched.  Stats: paths = sum of the owned counts, render_ms = the whole call.
+ * TCPT_ERR_INVALID: as tcpt_render_adaptive, a null buffer, row_offset >= row_stride (row_stride 0 = the whole frame). */
+int tcpt_render_adaptive_device(tcpt_ctx* ctx, const tcpt_render_params* params, const tcpt_adaptive_params* ap,
+                                void* dev_acc, void* dev_spp, void* stream);
 int tcpt_get_stats(const tcpt_ctx* ctx, tcpt_stats* out);
 
 /* ---- multi-GPU (SURVEY.md 8b / 8e).  The reference has no distributed path; every (pixel, sample) is independent and the only shared
@@ -222,6 +233,17 @@ int tcpt_shard_params(const tcpt_render_params* job, int shard_mode, int rank, i
 int tcpt_render_sharded(tcpt_ctx* ctx, const tcpt_render_params* job, int shard_mode, float* out_acc, float* out_srgb);
 /* same, accumulating into a caller-owned DEVICE buffer (zeroed by the caller) on `stream`; after the call rank 0's buffer holds the sum */
 int tcpt_render_sharded_device(tcpt_ctx* ctx, const tcpt_render_params* job, int shard_mode, void* dev_acc, void* stream);
+/* One complete ADAPTIVE frame (tcpt_render_adaptive) from all ranks.  Every rank passes the SAME whole-frame job (row_offset / row_stride,
+ * spp_begin / spp_end 0) and `ap`; rank r runs the rounds over its TILE shard alone (a rank without rows renders nothing but still joins
+ * the collective) with no collective per round: the rule reads only a pixel's own moments, so the frame -- accumulators, counts, sRGB --
+ * is BITWISE tcpt_render_adaptive's.  Then ONE grouped collective on the rendering stream: ncclReduce(sum) of the W*H*3 f32 accumulators
+ * and of the W*H u32 counts onto rank 0 (exact: every pixel not owned by a rank is +0 / 0 there).  Rank 0 applies the per-count output
+ * transform and makes one device -> host copy per requested buffer (out_acc, out_srgb, out_spp as in tcpt_render_adaptive; not all NULL);
+ * on the other ranks they may be NULL and are never written.  Stats as tcpt_render_adaptive over this rank's shard, reduce_ms as
+ * tcpt_render_sharded_device.  Without a communicator it is tcpt_render_adaptive.  No shard mode: the rule needs every sample of a pixel on
+ * one rank. */
+int tcpt_render_adaptive_sharded(tcpt_ctx* ctx, const tcpt_render_params* job, const tcpt_adaptive_params* ap,
+                                 float* out_acc, float* out_srgb, uint32_t* out_spp);
 
 typedef struct tcpt_group tcpt_group;
 int tcpt_group_create(const int* device_ids, int n, tcpt_group** out);     /* n contexts + one communicator clique */
@@ -232,6 +254,9 @@ const char* tcpt_group_last_error(const tcpt_group* g);
 int tcpt_group_set_tables(tcpt_group* g, const void* std_tables, size_t std_len, const float* rgb2spec, size_t rgb2spec_floats);
 int tcpt_group_build(tcpt_group* g, const float cam_pos[3]);               /* Scene::build on context 0, replica on every other GPU */
 int tcpt_group_render(tcpt_group* g, const tcpt_render_params* job, int shard_mode, float* out_acc, float* out_srgb);
+/* tcpt_render_adaptive_sharded on every GPU of the group, one host thread per GPU; out_* filled from device 0 */
+int tcpt_group_render_adaptive(tcpt_group* g, const tcpt_render_params* job, const tcpt_adaptive_params* ap,
+                               float* out_acc, float* out_srgb, uint32_t* out_spp);
 
 /* ---- synthetic triangle soups (BASELINE.json configs[4], 1 M - 100 M triangles): a TRAVERSAL-ONLY scene whose BVH is built on the device
  * (Morton order + radix tree, collapsed to the 4-wide records the traversal kernels read: csrc/lbvh.cuh; the reference's O(N^2) builder is

@@ -180,6 +180,8 @@ unsafe extern "C" {
                                 stream: *mut c_void) -> c_int;
     pub fn tcpt_render_adaptive(ctx: *mut TcptCtx, params: *const TcptRenderParams, ap: *const TcptAdaptiveParams, out_acc: *mut f32,
                                 out_srgb: *mut f32, out_spp: *mut u32) -> c_int;
+    pub fn tcpt_render_adaptive_device(ctx: *mut TcptCtx, params: *const TcptRenderParams, ap: *const TcptAdaptiveParams, dev_acc: *mut c_void,
+                                       dev_spp: *mut c_void, stream: *mut c_void) -> c_int;
     pub fn tcpt_get_stats(ctx: *const TcptCtx, out: *mut TcptStats) -> c_int;
 
     // multi-GPU: one context per GPU; the library owns the NCCL communicator (include/tcpt.h "multi-GPU")
@@ -189,6 +191,8 @@ unsafe extern "C" {
     pub fn tcpt_shard_params(job: *const TcptRenderParams, shard_mode: c_int, rank: c_int, nranks: c_int, out: *mut TcptRenderParams) -> c_int;
     pub fn tcpt_render_sharded(ctx: *mut TcptCtx, job: *const TcptRenderParams, shard_mode: c_int, out_acc: *mut f32, out_srgb: *mut f32) -> c_int;
     pub fn tcpt_render_sharded_device(ctx: *mut TcptCtx, job: *const TcptRenderParams, shard_mode: c_int, dev_acc: *mut c_void, stream: *mut c_void) -> c_int;
+    pub fn tcpt_render_adaptive_sharded(ctx: *mut TcptCtx, job: *const TcptRenderParams, ap: *const TcptAdaptiveParams, out_acc: *mut f32,
+                                        out_srgb: *mut f32, out_spp: *mut u32) -> c_int;
     // one host process, N GPUs: what GpuRendererImage::render_multi binds
     pub fn tcpt_group_create(device_ids: *const c_int, n: c_int, out: *mut *mut TcptGroup) -> c_int;
     pub fn tcpt_group_destroy(g: *mut TcptGroup);
@@ -198,6 +202,8 @@ unsafe extern "C" {
     pub fn tcpt_group_set_tables(g: *mut TcptGroup, std_tables: *const c_void, std_len: usize, rgb2spec: *const f32, rgb2spec_floats: usize) -> c_int;
     pub fn tcpt_group_build(g: *mut TcptGroup, cam_pos: *const f32) -> c_int;
     pub fn tcpt_group_render(g: *mut TcptGroup, job: *const TcptRenderParams, shard_mode: c_int, out_acc: *mut f32, out_srgb: *mut f32) -> c_int;
+    pub fn tcpt_group_render_adaptive(g: *mut TcptGroup, job: *const TcptRenderParams, ap: *const TcptAdaptiveParams, out_acc: *mut f32,
+                                      out_srgb: *mut f32, out_spp: *mut u32) -> c_int;
 }
 pub const TCPT_SHARD_TILE: c_int = 0;
 pub const TCPT_SHARD_SPP: c_int = 1;

@@ -207,6 +207,37 @@ impl GpuRendererImage {
             panic!("tcpt_group_render: {}", msg);
         }
     }
+    /// `render_adaptive` from every GPU of the communicator (`tcpt_render_adaptive_sharded`): each rank runs the rounds over its image
+    /// rows y % n == rank alone and ONE grouped reduce hands rank 0 the frame, bitwise the one-GPU `render_adaptive` frame. Every rank
+    /// calls it with the same image; `pixels`, `accumulators` and the returned sample counts are filled on rank 0 only.
+    pub fn render_adaptive_sharded<S: GpuSampler>(&mut self, threshold: f32, min_spp: u32, step: u32) -> Vec<u32> {
+        self.params.sampler = S::ID;
+        let ap = TcptAdaptiveParams { threshold, min_spp, step };
+        let mut counts = vec![0u32; (self.params.width * self.params.height) as usize];
+        let rc = unsafe {
+            tcpt_render_adaptive_sharded(self.ctx, &self.params, &ap, self.accumulators.as_mut_ptr() as *mut f32,
+                                         self.pixels.as_mut_ptr() as *mut f32, counts.as_mut_ptr())
+        };
+        if rc != TCPT_OK {
+            panic!("tcpt_render_adaptive_sharded: {}", last_error(self.ctx));
+        }
+        counts
+    }
+    /// The same from ONE host process that owns all GPUs of the box (`tcpt_group_render_adaptive`); returns the sample counts.
+    pub fn render_group_adaptive<S: GpuSampler>(&mut self, group: *mut TcptGroup, threshold: f32, min_spp: u32, step: u32) -> Vec<u32> {
+        self.params.sampler = S::ID;
+        let ap = TcptAdaptiveParams { threshold, min_spp, step };
+        let mut counts = vec![0u32; (self.params.width * self.params.height) as usize];
+        let rc = unsafe {
+            tcpt_group_render_adaptive(group, &self.params, &ap, self.accumulators.as_mut_ptr() as *mut f32, self.pixels.as_mut_ptr() as *mut f32,
+                                       counts.as_mut_ptr())
+        };
+        if rc != TCPT_OK {
+            let msg = unsafe { std::ffi::CStr::from_ptr(tcpt_group_last_error(group)) }.to_string_lossy().into_owned();
+            panic!("tcpt_group_render_adaptive: {}", msg);
+        }
+        counts
+    }
     pub fn stats(&self) -> TcptStats {
         let mut s = TcptStats::default();
         unsafe { tcpt_get_stats(self.ctx, &mut s) };

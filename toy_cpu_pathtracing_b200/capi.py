@@ -79,7 +79,7 @@ EXPORTED_SYMBOLS = [
     "tcpt_create", "tcpt_destroy", "tcpt_last_error", "tcpt_set_option", "tcpt_set_tables", "tcpt_scene_clear",
     "tcpt_scene_add_mesh", "tcpt_scene_add_single_triangle", "tcpt_scene_add_texture", "tcpt_scene_add_material", "tcpt_scene_add_primitive",
     "tcpt_scene_add_env_light", "tcpt_scene_add_delta_light", "tcpt_scene_build", "tcpt_render", "tcpt_render_device", "tcpt_finalize_device",
-    "tcpt_render_adaptive",
+    "tcpt_render_adaptive", "tcpt_render_adaptive_device", "tcpt_render_adaptive_sharded", "tcpt_group_render_adaptive",
     "tcpt_get_stats", "tcpt_trace", "tcpt_trace_device", "tcpt_sampler_stream", "tcpt_path_samples", "tcpt_get_bvh",
     "tcpt_get_wide_bvh", "tcpt_build_bvh_boxes", "tcpt_rgb_to_coeffs", "tcpt_get_mesh_tangents", "tcpt_upload_flat_scene",
     "tcpt_comm_get_unique_id", "tcpt_comm_init", "tcpt_comm_destroy", "tcpt_shard_params", "tcpt_render_sharded", "tcpt_render_sharded_device",
@@ -115,6 +115,9 @@ def load_library() -> C.CDLL:
         "tcpt_render_device": (I, [P, C.POINTER(RenderParams), C.c_void_p, C.c_void_p]),
         "tcpt_finalize_device": (I, [P, C.c_void_p, U, U, U, C.c_void_p, C.c_void_p]),
         "tcpt_render_adaptive": (I, [P, C.POINTER(RenderParams), C.POINTER(AdaptiveParams), fp, fp, up]),
+        "tcpt_render_adaptive_device": (I, [P, C.POINTER(RenderParams), C.POINTER(AdaptiveParams), C.c_void_p, C.c_void_p, C.c_void_p]),
+        "tcpt_render_adaptive_sharded": (I, [P, C.POINTER(RenderParams), C.POINTER(AdaptiveParams), fp, fp, up]),
+        "tcpt_group_render_adaptive": (I, [P, C.POINTER(RenderParams), C.POINTER(AdaptiveParams), fp, fp, up]),
         "tcpt_get_stats": (I, [P, C.POINTER(Stats)]), "tcpt_trace": (I, [P, fp, I, I, ip]),
         "tcpt_trace_device": (I, [P, C.c_void_p, I, I, C.c_void_p, C.c_void_p]),
         "tcpt_sampler_stream": (I, [P, I, U, U, U, U, U, U, U, ip, I, fp]),

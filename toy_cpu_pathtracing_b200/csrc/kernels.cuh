@@ -28,7 +28,7 @@ namespace tcpt {
 struct PathList { const uint32_t* xy; const uint32_t* sample; };  // explicit (pixel, sample) lists for tcpt_path_samples
 
 // owned pixel index of pass pixel p_local: consecutive from pix_begin, or the pix_begin + p_local-th entry of the pass's pixel list
-// (adaptive rounds: the frame indices of the pixels still active, in ascending order)
+// (adaptive rounds: the owned indices of the pixels still active, in ascending order; the frame index for a whole-frame job)
 __device__ __forceinline__ uint32_t owned_pixel(const DRender& R, uint32_t p_local) {
     return R.pix_list ? __ldg(R.pix_list + R.pix_begin + p_local) : R.pix_begin + p_local;
 }
@@ -906,17 +906,29 @@ __device__ __forceinline__ uint32_t block_exclusive_scan(uint32_t v, uint32_t* t
     return excl;
 }
 
-// this thread's entries of the active list (nullptr = the identity list 0 .. n - 1): frame pixel indices and the mask of the ones that stay active
+// The rows of a job (DRender::row_offset / row_stride) and the exact division by the width (DRender::width_magic): owned pixel index ->
+// frame pixel index, the index of the per-pixel tables (moments, counts)
+struct RowMap {
+    uint32_t width, row_offset, row_stride; uint64_t width_magic;
+    __device__ __forceinline__ uint32_t frame_pixel(uint32_t k) const {
+        const uint32_t row = div_magic(k, width_magic);
+        return (row_offset + row * row_stride) * width + (k - row * width);
+    }
+};
+
+// this thread's entries of the active list (nullptr = the identity list 0 .. n - 1): owned indices, their frame indices and the mask of
+// the ones that stay active
 __device__ __forceinline__ uint32_t adaptive_items(const uint32_t* __restrict__ list, uint32_t n, const float2* __restrict__ mom, uint32_t k, float threshold,
-                                                   uint32_t pix[TCPT_SELECT_ITEMS], uint32_t* valid) {
+                                                   const RowMap& rm, uint32_t own[TCPT_SELECT_ITEMS], uint32_t pix[TCPT_SELECT_ITEMS], uint32_t* valid) {
     const uint32_t first = (blockIdx.x * TCPT_SELECT_THREADS + threadIdx.x) * TCPT_SELECT_ITEMS;
     uint32_t keep = 0u, ok = 0u;
 #pragma unroll
     for (uint32_t j = 0; j < TCPT_SELECT_ITEMS; ++j) {
         const uint32_t i = first + j;
-        pix[j] = 0u;
+        own[j] = pix[j] = 0u;
         if (i >= n) continue;
-        pix[j] = list ? list[i] : i;
+        own[j] = list ? list[i] : i;
+        pix[j] = rm.frame_pixel(own[j]);
         ok |= 1u << j;
         if (!adaptive_converged(mom[pix[j]], k, threshold)) keep |= 1u << j;
     }
@@ -924,11 +936,12 @@ __device__ __forceinline__ uint32_t adaptive_items(const uint32_t* __restrict__ 
     return keep;
 }
 
-// count: every pixel that stops gets its sample count k; tile_counts[tile] = survivors of the tile
+// count: every pixel that stops gets its sample count k (at its frame index); tile_counts[tile] = survivors of the tile
 __global__ void __launch_bounds__(TCPT_SELECT_THREADS) k_adaptive_count(const uint32_t* __restrict__ list, uint32_t n, const float2* __restrict__ mom,
-                                                                        uint32_t k, float threshold, uint32_t* __restrict__ counts, uint32_t* __restrict__ tile_counts) {
-    uint32_t pix[TCPT_SELECT_ITEMS], valid;
-    const uint32_t keep = adaptive_items(list, n, mom, k, threshold, pix, &valid);
+                                                                        uint32_t k, float threshold, const RowMap rm, uint32_t* __restrict__ counts,
+                                                                        uint32_t* __restrict__ tile_counts) {
+    uint32_t own[TCPT_SELECT_ITEMS], pix[TCPT_SELECT_ITEMS], valid;
+    const uint32_t keep = adaptive_items(list, n, mom, k, threshold, rm, own, pix, &valid);
 #pragma unroll
     for (uint32_t j = 0; j < TCPT_SELECT_ITEMS; ++j)
         if (((valid & ~keep) >> j) & 1u) counts[pix[j]] = k;
@@ -951,16 +964,18 @@ __global__ void __launch_bounds__(1024) k_adaptive_scan(uint32_t* __restrict__ t
     if (threadIdx.x == 0) *n_out = carry;
 }
 
-// scatter: the survivors of every tile to list_out from the tile's offset, in list order (the rule is evaluated again: same inputs, same answer)
+// scatter: the owned indices of every tile's survivors to list_out from the tile's offset, in list (ascending) order (the rule is evaluated
+// again: same inputs, same answer)
 __global__ void __launch_bounds__(TCPT_SELECT_THREADS) k_adaptive_scatter(const uint32_t* __restrict__ list, uint32_t n, const float2* __restrict__ mom,
-                                                                          uint32_t k, float threshold, const uint32_t* __restrict__ tile_offsets, uint32_t* __restrict__ list_out) {
-    uint32_t pix[TCPT_SELECT_ITEMS], valid;
-    const uint32_t keep = adaptive_items(list, n, mom, k, threshold, pix, &valid);
+                                                                          uint32_t k, float threshold, const RowMap rm, const uint32_t* __restrict__ tile_offsets,
+                                                                          uint32_t* __restrict__ list_out) {
+    uint32_t own[TCPT_SELECT_ITEMS], pix[TCPT_SELECT_ITEMS], valid;
+    const uint32_t keep = adaptive_items(list, n, mom, k, threshold, rm, own, pix, &valid);
     uint32_t total;
     uint32_t o = tile_offsets[blockIdx.x] + block_exclusive_scan((uint32_t)__popc(keep), &total);
 #pragma unroll
     for (uint32_t j = 0; j < TCPT_SELECT_ITEMS; ++j)
-        if ((keep >> j) & 1u) list_out[o++] = pix[j];
+        if ((keep >> j) & 1u) list_out[o++] = own[j];
 }
 
 // k_finalize mode 0 with a per-pixel divisor: the value of a pixel with count k is bitwise what k_finalize gives with spp = k
@@ -974,8 +989,9 @@ __global__ void __launch_bounds__(256) k_finalize_counts(const float* __restrict
     }
 }
 
-__global__ void __launch_bounds__(256) k_fill_u32(uint32_t* __restrict__ p, uint32_t n, uint32_t value) {
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) p[i] = value;
+// p[frame pixel of owned index i] = value for the n owned pixels of a job; no other entry of p is written
+__global__ void __launch_bounds__(256) k_fill_owned_u32(uint32_t* __restrict__ p, uint32_t n, const RowMap rm, uint32_t value) {
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) p[rm.frame_pixel(i)] = value;
 }
 
 // ---------------------------------------------------------------- single-stage probes for parity tests and the traversal micro-benchmark

@@ -211,10 +211,12 @@ int grid_for(const tcpt_ctx* ctx, uint64_t n, int block) {
 uint32_t log2_int(uint32_t v) { return v == 0 ? 0 : 31 - (uint32_t)__builtin_clz(v); }
 uint32_t round_up_pow2(uint32_t v) { return v <= 1 ? 1u : 1u << (32 - __builtin_clz(v - 1)); }
 
+// the multiplier of div_magic for the divisor d
+uint64_t div_magic_of(uint32_t d) { return d <= 1u ? 0ull : (~0ull) / d + 1ull; }   // floor((2^64 - 1) / d) + 1 == floor(2^64 / d) + 1 unless d divides 2^64: then one more than that, still exact (n / 2^64 < 1 / d)
+
 // DRender::n_pix_magic / width_magic (see div_magic): call after n_pix and width are set
 void set_div_magics(DRender& R) {
-    auto magic = [](uint32_t d) -> uint64_t { return d <= 1u ? 0ull : (~0ull) / d + 1ull; };   // floor((2^64 - 1) / d) + 1 == floor(2^64 / d) + 1 unless d divides 2^64: then one more than that, still exact (n / 2^64 < 1 / d)
-    R.n_pix_magic = magic(R.n_pix); R.width_magic = magic(R.width);
+    R.n_pix_magic = div_magic_of(R.n_pix); R.width_magic = div_magic_of(R.width);
 }
 
 int make_render(tcpt_ctx* ctx, const tcpt_render_params* p, DRender& R, DCamera& cam) {
@@ -483,8 +485,8 @@ void reset_stats(tcpt_ctx* ctx) {
     ctx->ev_used = 0; ctx->ev_stage.clear();
 }
 
-// The pass loop of a job: `owned` pixels -- owned indices 0 .. owned - 1, or the entries of the device list `pix_list` (frame indices of a
-// job with row_offset 0 / row_stride 1) -- times the sample window [s0, s1), cut into (pixel block x sample window) passes that fit the
+// The pass loop of a job: `owned` pixels -- owned indices 0 .. owned - 1, or the entries of the device list `pix_list` (owned indices,
+// ascending; see owned_pixel) -- times the sample window [s0, s1), cut into (pixel block x sample window) passes that fit the
 // path-slot budget.  R comes from make_render + ensure_sobol_prefix.  dev_mom != nullptr: the film also adds the luminance moments.
 int render_passes(tcpt_ctx* ctx, const DRender& R, const DCamera& cam, uint64_t owned, const uint32_t* pix_list, uint32_t s0, uint32_t s1,
                   uint32_t max_slots, float* dev_acc, float2* dev_mom, cudaStream_t stream) {
@@ -583,7 +585,7 @@ int ensure_film(tcpt_ctx* ctx, size_t n) {
     return TCPT_OK;
 }
 
-// tcpt_render_adaptive's per-pixel buffers, carved from one grow-only allocation
+// the adaptive entry points' per-pixel buffers, carved from one grow-only allocation
 struct AdaptiveBuffers { float2* mom; uint32_t* counts; uint32_t* list[2]; uint32_t* tiles; uint32_t* n_active; };
 size_t adaptive_bytes(size_t n_pix) { return n_pix * (sizeof(float2) + 3 * sizeof(uint32_t)) + ((n_pix + TCPT_SELECT_TILE - 1) / TCPT_SELECT_TILE + 1) * sizeof(uint32_t); }
 int ensure_adaptive(tcpt_ctx* ctx, size_t n_pix, AdaptiveBuffers& b) {
@@ -599,6 +601,110 @@ int ensure_adaptive(tcpt_ctx* ctx, size_t n_pix, AdaptiveBuffers& b) {
     b.list[0] = b.counts + cap; b.list[1] = b.list[0] + cap;
     b.n_active = b.list[1] + cap;
     b.tiles = b.n_active + 1;
+    return TCPT_OK;
+}
+
+// The checks every adaptive entry point makes on `ap` and the job before it looks at the device (include/tcpt.h).  The row shard is the
+// caller's to check: each entry point has its own rule.
+int check_adaptive(tcpt_ctx* ctx, const tcpt_render_params* p, const tcpt_adaptive_params* ap, const char* who) {
+    auto bad = [&](const char* why) { return fail(ctx, TCPT_ERR_INVALID, std::string(who) + ": " + why); };
+    if (!std::isfinite(ap->threshold) || ap->threshold < 0.0f) return bad("threshold must be finite and >= 0");
+    if (ap->min_spp < 2 || ap->min_spp > p->spp) return bad("min_spp must lie in [2, spp]");
+    if (ap->step == 0) return bad("step must be positive");
+    if (p->integrator < TCPT_INTEGRATOR_PT || p->integrator > TCPT_INTEGRATOR_MIS) return bad("integrators pt, nee and mis only");
+    if (p->spp_begin || p->spp_end) return bad("spp_begin / spp_end must be 0 (all samples)");
+    if ((uint64_t)p->width * p->height * 3 > 0xffffffffull) return bad("frame too large");
+    return TCPT_OK;
+}
+
+// The adaptive rounds of one job on `s`: the whole frame, or the rows row_offset + i * row_stride.  R / cam come from make_render of `p`,
+// which the caller runs before it records anything on the device; the caller also checks the row shard (row_offset < row_stride).  Round 0 takes
+// every owned pixel (no list); after each round that ends below spp, k_adaptive_count / _scan / _scatter write the counts of the pixels that
+// stop and compact the others, in ascending owned order, into the next list.  One 4-byte device -> host copy per round (the active count)
+// sizes the next round.  Each owned pixel's sum is ADDED into dev_acc and its count WRITTEN into dev_counts (both frame-indexed, W*H*3 f32
+// and W*H u32); no other pixel of either buffer is touched.
+int render_adaptive_into(tcpt_ctx* ctx, const tcpt_render_params* p, DRender R, const DCamera& cam, const tcpt_adaptive_params* ap, float* dev_acc,
+                         uint32_t* dev_counts, cudaStream_t s) {
+    int rc;
+    const uint32_t n_pix = p->width * p->height, N = p->spp;
+    const uint32_t rows = R.row_offset < p->height ? (p->height - R.row_offset + R.row_stride - 1) / R.row_stride : 0;
+    const uint32_t owned = rows * p->width;
+    AdaptiveBuffers B;
+    if ((rc = ensure_adaptive(ctx, n_pix, B)) != TCPT_OK) return rc;
+    if (owned == 0) return TCPT_OK;
+    if ((rc = ensure_sobol_prefix(ctx, R, s)) != TCPT_OK) return rc;
+    const RowMap rm{R.width, R.row_offset, R.row_stride, div_magic_of(R.width)};
+    CU(cudaMemsetAsync(B.mom, 0, (size_t)n_pix * sizeof(float2), s));
+    k_fill_owned_u32<<<grid_for(ctx, owned, 256), 256, 0, s>>>(dev_counts, owned, rm, N);   // a pixel that never stops has count N
+    ctx->stats.kernel_launches++;
+    uint32_t k = 0, active = owned, cur = 0;
+    const uint32_t* list = nullptr;   // round 0: every owned pixel, in order
+    while (active > 0) {
+        const uint64_t want = k == 0 ? ap->min_spp : (uint64_t)k + ap->step;
+        const uint32_t k_next = want < N ? (uint32_t)want : N;
+        if ((rc = render_passes(ctx, R, cam, active, list, k, k_next, p->max_slots, dev_acc, B.mom, s)) != TCPT_OK) return rc;
+        k = k_next;
+        if (k >= N) break;
+        const uint32_t n_tiles = (active + TCPT_SELECT_TILE - 1) / TCPT_SELECT_TILE;
+        k_adaptive_count<<<n_tiles, TCPT_SELECT_THREADS, 0, s>>>(list, active, B.mom, k, ap->threshold, rm, dev_counts, B.tiles);
+        k_adaptive_scan<<<1, 1024, 0, s>>>(B.tiles, n_tiles, B.n_active);
+        k_adaptive_scatter<<<n_tiles, TCPT_SELECT_THREADS, 0, s>>>(list, active, B.mom, k, ap->threshold, rm, B.tiles, B.list[cur]);
+        ctx->stats.kernel_launches += 3;
+        CU(cudaGetLastError());
+        CU(cudaMemcpyAsync(&active, B.n_active, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+        CU(cudaStreamSynchronize(s));
+        list = B.list[cur]; cur ^= 1u;
+    }
+    return TCPT_OK;
+}
+
+// One adaptive frame on the context's stream: `mine` (the whole job, or this rank's tile shard of it) through render_adaptive_into into the
+// context's film and count buffers.  collective = false: the frame is this context's alone (any communicator it has is not used) and it
+// finalizes and copies out.  collective = true (tcpt_render_adaptive_sharded): with a communicator of more than one rank, ONE grouped
+// collective then sums both buffers onto rank 0 (exact: every pixel is owned by one rank, the others hold +0 and 0); rank 0 finalizes and
+// copies out, the other ranks write no host buffer.
+int adaptive_frame(tcpt_ctx* ctx, const tcpt_render_params* mine, const tcpt_adaptive_params* ap, bool collective, float* out_acc, float* out_srgb,
+                   uint32_t* out_spp) {
+    const uint32_t n_pix = mine->width * mine->height;
+    const size_t n = (size_t)n_pix * 3;
+    const bool reduce = collective && ctx->comm_size > 1, root = !collective || ctx->comm_rank == 0;
+    cudaStream_t s = ctx->stream;
+    DRender R; DCamera cam;
+    int rc = make_render(ctx, mine, R, cam);
+    if (rc) return rc;
+    AdaptiveBuffers B;
+    if ((rc = ensure_film(ctx, n)) != TCPT_OK || (rc = ensure_adaptive(ctx, n_pix, B)) != TCPT_OK) return rc;
+    reset_stats(ctx);
+    CU(cudaEventRecord(ctx->ev0, s));
+    CU(cudaMemsetAsync(ctx->film_acc, 0, n * sizeof(float), s));
+    if (reduce) CU(cudaMemsetAsync(B.counts, 0, (size_t)n_pix * sizeof(uint32_t), s));   // the pixels of the other ranks
+    if ((rc = render_adaptive_into(ctx, mine, R, cam, ap, ctx->film_acc, B.counts, s)) != TCPT_OK) return rc;
+    if (reduce) {
+        if (!ctx->ev_r0) { cudaEventCreate(&ctx->ev_r0); cudaEventCreate(&ctx->ev_r1); }
+        CU(cudaEventRecord(ctx->ev_r0, s));
+        g_nccl.GroupStart();
+        const ncclResult_t ra = g_nccl.Reduce(ctx->film_acc, ctx->film_acc, n, ncclFloat32, ncclSum, 0, ctx->comm, s);
+        const ncclResult_t rb = g_nccl.Reduce(B.counts, B.counts, n_pix, ncclUint32, ncclSum, 0, ctx->comm, s);
+        const ncclResult_t re = g_nccl.GroupEnd();
+        const ncclResult_t r = ra != ncclSuccess ? ra : rb != ncclSuccess ? rb : re;
+        if (r != ncclSuccess) return fail(ctx, TCPT_ERR_CUDA, std::string("ncclReduce: ") + g_nccl.GetErrorString(r));
+        CU(cudaEventRecord(ctx->ev_r1, s));
+    }
+    if (root && out_srgb) {
+        k_finalize_counts<<<grid_for(ctx, n, 256), 256, 0, s>>>(ctx->film_acc, B.counts, ctx->film_srgb, (uint32_t)n);
+        ctx->stats.kernel_launches++;
+        CU(cudaGetLastError());
+    }
+    CU(cudaEventRecord(ctx->ev1, s));
+    CU(cudaEventSynchronize(ctx->ev1));
+    float ms = 0; CU(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+    ctx->stats.render_ms = ms;
+    if (reduce) { float rms = 0; if (cudaEventElapsedTime(&rms, ctx->ev_r0, ctx->ev_r1) == cudaSuccess) ctx->stats.reduce_ms = rms; }
+    collect_stage_times(ctx);
+    if ((rc = fetch_stats(ctx)) != TCPT_OK || !root) return rc;
+    if (out_acc && (rc = copy_out(ctx, 0, out_acc, ctx->film_acc, n * sizeof(float))) != TCPT_OK) return rc;
+    if (out_srgb && (rc = copy_out(ctx, 1, out_srgb, ctx->film_srgb, n * sizeof(float))) != TCPT_OK) return rc;
+    if (out_spp && (rc = copy_out(ctx, 2, out_spp, B.counts, (size_t)n_pix * sizeof(uint32_t))) != TCPT_OK) return rc;
     return TCPT_OK;
 }
 
@@ -1133,70 +1239,40 @@ int tcpt_render(tcpt_ctx* ctx, const tcpt_render_params* params, float* out_acc,
     return TCPT_OK;
 }
 
-// Adaptive sampling (include/tcpt.h): rounds of render_passes over the pixels still active.  Round 0 takes every pixel (no list); after
-// each round that ends below spp, k_adaptive_count / _scan / _scatter write the counts of the pixels that stop and compact the others,
-// in ascending pixel order, into the next list.  One 4-byte device -> host copy per round (the active count) sizes the next round.
+// Adaptive sampling (include/tcpt.h): the whole frame through adaptive_frame / render_adaptive_into.
 int tcpt_render_adaptive(tcpt_ctx* ctx, const tcpt_render_params* params, const tcpt_adaptive_params* ap, float* out_acc, float* out_srgb, uint32_t* out_spp) {
     if (!ctx || !params || !ap) return TCPT_ERR_INVALID;
     if (!out_acc && !out_srgb && !out_spp) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive: no output buffer");
-    if (!std::isfinite(ap->threshold) || ap->threshold < 0.0f) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive: threshold must be finite and >= 0");
-    if (ap->min_spp < 2 || ap->min_spp > params->spp) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive: min_spp must lie in [2, spp]");
-    if (ap->step == 0) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive: step must be positive");
-    if (params->integrator < TCPT_INTEGRATOR_PT || params->integrator > TCPT_INTEGRATOR_MIS) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive: integrators pt, nee and mis only");
+    int rc = check_adaptive(ctx, params, ap, "render_adaptive");
+    if (rc) return rc;
     if (params->row_offset || params->row_stride) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive: row_offset / row_stride must be 0 (whole frame)");
-    if (params->spp_begin || params->spp_end) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive: spp_begin / spp_end must be 0 (all samples)");
     if (!ctx->stream) return fail(ctx, TCPT_ERR_CUDA, "no CUDA device");
     CU(cudaSetDevice(ctx->device));
-    DRender R; DCamera cam;
-    int rc = make_render(ctx, params, R, cam);
+    return adaptive_frame(ctx, params, ap, false, out_acc, out_srgb, out_spp);
+}
+
+// One row shard of an adaptive job into the caller's device buffers, on the caller's stream; no collective.
+int tcpt_render_adaptive_device(tcpt_ctx* ctx, const tcpt_render_params* params, const tcpt_adaptive_params* ap, void* dev_acc, void* dev_spp, void* stream) {
+    if (!ctx || !params || !ap) return TCPT_ERR_INVALID;
+    if (!dev_acc || !dev_spp) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive_device: dev_acc and dev_spp are required");
+    int rc = check_adaptive(ctx, params, ap, "render_adaptive_device");
     if (rc) return rc;
-    const uint64_t n_pix64 = (uint64_t)params->width * params->height;
-    if (n_pix64 * 3 > 0xffffffffull) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive: frame too large");
-    const uint32_t n_pix = (uint32_t)n_pix64, N = params->spp;
-    const size_t n = (size_t)n_pix * 3;
-    cudaStream_t s = ctx->stream;
-    AdaptiveBuffers B;
-    if ((rc = ensure_film(ctx, n)) != TCPT_OK || (rc = ensure_adaptive(ctx, n_pix, B)) != TCPT_OK) return rc;
+    if (params->row_offset && params->row_offset >= params->row_stride) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive_device: row_offset must be < row_stride");
+    if (!ctx->stream) return fail(ctx, TCPT_ERR_CUDA, "no CUDA device");
+    CU(cudaSetDevice(ctx->device));
+    cudaStream_t s = stream ? (cudaStream_t)stream : ctx->stream;
+    DRender R; DCamera cam;
+    if ((rc = make_render(ctx, params, R, cam)) != TCPT_OK) return rc;
     reset_stats(ctx);
+    if (s != ctx->stream) CU(cudaStreamSynchronize(ctx->stream));
     CU(cudaEventRecord(ctx->ev0, s));
-    if ((rc = ensure_sobol_prefix(ctx, R, s)) != TCPT_OK) return rc;
-    CU(cudaMemsetAsync(ctx->film_acc, 0, n * sizeof(float), s));
-    CU(cudaMemsetAsync(B.mom, 0, (size_t)n_pix * sizeof(float2), s));
-    k_fill_u32<<<grid_for(ctx, n_pix, 256), 256, 0, s>>>(B.counts, n_pix, N);   // a pixel that never stops has count N
-    ctx->stats.kernel_launches++;
-    uint32_t k = 0, active = n_pix, cur = 0;
-    const uint32_t* list = nullptr;   // round 0: every pixel, in order
-    while (active > 0) {
-        const uint64_t want = k == 0 ? ap->min_spp : (uint64_t)k + ap->step;
-        const uint32_t k_next = want < N ? (uint32_t)want : N;
-        if ((rc = render_passes(ctx, R, cam, active, list, k, k_next, params->max_slots, ctx->film_acc, B.mom, s)) != TCPT_OK) return rc;
-        k = k_next;
-        if (k >= N) break;
-        const uint32_t n_tiles = (active + TCPT_SELECT_TILE - 1) / TCPT_SELECT_TILE;
-        k_adaptive_count<<<n_tiles, TCPT_SELECT_THREADS, 0, s>>>(list, active, B.mom, k, ap->threshold, B.counts, B.tiles);
-        k_adaptive_scan<<<1, 1024, 0, s>>>(B.tiles, n_tiles, B.n_active);
-        k_adaptive_scatter<<<n_tiles, TCPT_SELECT_THREADS, 0, s>>>(list, active, B.mom, k, ap->threshold, B.tiles, B.list[cur]);
-        ctx->stats.kernel_launches += 3;
-        CU(cudaGetLastError());
-        CU(cudaMemcpyAsync(&active, B.n_active, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-        CU(cudaStreamSynchronize(s));
-        list = B.list[cur]; cur ^= 1u;
-    }
-    if (out_srgb) {
-        k_finalize_counts<<<grid_for(ctx, n, 256), 256, 0, s>>>(ctx->film_acc, B.counts, ctx->film_srgb, (uint32_t)n);
-        ctx->stats.kernel_launches++;
-        CU(cudaGetLastError());
-    }
+    if ((rc = render_adaptive_into(ctx, params, R, cam, ap, (float*)dev_acc, (uint32_t*)dev_spp, s)) != TCPT_OK) return rc;
     CU(cudaEventRecord(ctx->ev1, s));
     CU(cudaEventSynchronize(ctx->ev1));
     float ms = 0; CU(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
     ctx->stats.render_ms = ms;
     collect_stage_times(ctx);
-    if ((rc = fetch_stats(ctx)) != TCPT_OK) return rc;
-    if (out_acc && (rc = copy_out(ctx, 0, out_acc, ctx->film_acc, n * sizeof(float))) != TCPT_OK) return rc;
-    if (out_srgb && (rc = copy_out(ctx, 1, out_srgb, ctx->film_srgb, n * sizeof(float))) != TCPT_OK) return rc;
-    if (out_spp && (rc = copy_out(ctx, 2, out_spp, B.counts, (size_t)n_pix * sizeof(uint32_t))) != TCPT_OK) return rc;
-    return TCPT_OK;
+    return fetch_stats(ctx);
 }
 
 // ---------------------------------------------------------------- multi-GPU: NCCL inside the library (SURVEY.md 8b / 8e)
@@ -1311,6 +1387,24 @@ int tcpt_render_sharded(tcpt_ctx* ctx, const tcpt_render_params* job, int shard_
     return TCPT_OK;
 }
 
+// One complete adaptive frame from all ranks: rank r runs the rounds over its tile shard alone (the stopping rule reads only a pixel's own
+// moments, so every pixel stops where it stops on one GPU) and the ranks meet once, in adaptive_frame's grouped reduce.
+int tcpt_render_adaptive_sharded(tcpt_ctx* ctx, const tcpt_render_params* job, const tcpt_adaptive_params* ap, float* out_acc, float* out_srgb, uint32_t* out_spp) {
+    if (!ctx || !job || !ap) return TCPT_ERR_INVALID;
+    const bool root = ctx->comm_rank == 0;
+    if (root && !out_acc && !out_srgb && !out_spp) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive_sharded: no output buffer on rank 0");
+    int rc = check_adaptive(ctx, job, ap, "render_adaptive_sharded");
+    if (rc) return rc;
+    if (job->row_offset || job->row_stride) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive_sharded: the job describes the whole frame (row_offset / row_stride 0)");
+    if (!ctx->stream) return fail(ctx, TCPT_ERR_CUDA, "no CUDA device");
+    if (ctx->comm_size > 1 && !ctx->comm) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive_sharded: call tcpt_comm_init first");
+    CU(cudaSetDevice(ctx->device));
+    tcpt_render_params mine;
+    if (tcpt_shard_params(job, TCPT_SHARD_TILE, ctx->comm_rank, ctx->comm_size, &mine) != TCPT_OK) return fail(ctx, TCPT_ERR_INVALID, "render_adaptive_sharded: bad job");
+    mine.spp_begin = mine.spp_end = 0;   // every sample of the owned rows
+    return adaptive_frame(ctx, &mine, ap, true, root ? out_acc : nullptr, root ? out_srgb : nullptr, root ? out_spp : nullptr);
+}
+
 
 // ---------------------------------------------------------------- one host process, several GPUs (the shape a Rust `GpuRendererImage` would use)
 struct tcpt_group {
@@ -1383,17 +1477,33 @@ int tcpt_group_build(tcpt_group* g, const float cam_pos[3]) {
     return TCPT_OK;
 }
 
-// One complete frame from all GPUs of the group: one host thread per GPU (tcpt_render_sharded), out_* filled from device 0.
-int tcpt_group_render(tcpt_group* g, const tcpt_render_params* job, int shard_mode, float* out_acc, float* out_srgb) {
-    if (!g || g->ctx.empty() || !job || (!out_acc && !out_srgb)) return TCPT_ERR_INVALID;
+// render(ctx, root) on every context of the group, one host thread per GPU; root = whether ctx is device 0, the one whose out_* are filled
+extern "C++" {
+template <class F>
+static int group_each(tcpt_group* g, F render) {
     const size_t n = g->ctx.size();
     std::vector<int> rcs(n, TCPT_OK);
     std::vector<std::thread> th;
-    for (size_t i = 1; i < n; ++i) th.emplace_back([&, i] { rcs[i] = tcpt_render_sharded(g->ctx[i], job, shard_mode, nullptr, nullptr); });
-    rcs[0] = tcpt_render_sharded(g->ctx[0], job, shard_mode, out_acc, out_srgb);
+    for (size_t i = 1; i < n; ++i) th.emplace_back([&, i] { rcs[i] = render(g->ctx[i], false); });
+    rcs[0] = render(g->ctx[0], true);
     for (auto& t : th) t.join();
     for (size_t i = 0; i < n; ++i) if (rcs[i]) { g->error = g->ctx[i]->error; return rcs[i]; }
     return TCPT_OK;
+}
+}
+
+// One complete frame from all GPUs of the group: one host thread per GPU (tcpt_render_sharded), out_* filled from device 0.
+int tcpt_group_render(tcpt_group* g, const tcpt_render_params* job, int shard_mode, float* out_acc, float* out_srgb) {
+    if (!g || g->ctx.empty() || !job || (!out_acc && !out_srgb)) return TCPT_ERR_INVALID;
+    return group_each(g, [&](tcpt_ctx* c, bool root) { return tcpt_render_sharded(c, job, shard_mode, root ? out_acc : nullptr, root ? out_srgb : nullptr); });
+}
+
+// The same for an adaptive frame (tcpt_render_adaptive_sharded on every GPU).
+int tcpt_group_render_adaptive(tcpt_group* g, const tcpt_render_params* job, const tcpt_adaptive_params* ap, float* out_acc, float* out_srgb, uint32_t* out_spp) {
+    if (!g || g->ctx.empty() || !job || !ap || (!out_acc && !out_srgb && !out_spp)) return TCPT_ERR_INVALID;
+    return group_each(g, [&](tcpt_ctx* c, bool root) {
+        return tcpt_render_adaptive_sharded(c, job, ap, root ? out_acc : nullptr, root ? out_srgb : nullptr, root ? out_spp : nullptr);
+    });
 }
 
 int tcpt_get_stats(const tcpt_ctx* ctx, tcpt_stats* out) {

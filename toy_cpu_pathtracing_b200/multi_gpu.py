@@ -12,6 +12,8 @@ there.  torch.distributed is only the plumbing that carries the 128-byte NCCL un
                sample order on one GPU, other ranks contribute exact zeros: the reduced film is bitwise equal to 1 GPU.
   mode "spp" : rank r renders samples [r*spp/world, (r+1)*spp/world) of every pixel -> best balance; per-pixel float sums are
                re-associated across ranks (tolerance-level equality).
+
+Adaptive frames (`RendererImage.render_adaptive_sharded`, tcpt_render_adaptive_sharded) take tile shards only, one grouped reduce per frame.
 """
 from __future__ import annotations
 

@@ -111,6 +111,12 @@ class NormalRenderer(_SrgbRenderer):   # renderer/src/renderer/normal_renderer.r
 RENDERERS = {"pt": SrgbRendererPt, "nee": SrgbRendererNee, "mis": SrgbRendererMis, "albedo": AlbedoRenderer, "normal": NormalRenderer}
 
 
+def _rounds(sample_counts, min_spp, step) -> int:
+    """Rounds an adaptive frame took.  The last round ends at the largest count: round 0 reaches min_spp, every later one `step` more
+    (the last clipped at spp)."""
+    return 1 + -(-(int(sample_counts.max()) - int(min_spp)) // int(step))
+
+
 class RendererImage:                  # renderer/src/renderer.rs:101-149
     def __init__(self, width: int, height: int, renderer: _SrgbRenderer):
         self.width, self.height, self.renderer = int(width), int(height), renderer
@@ -155,8 +161,32 @@ class RendererImage:                  # renderer/src/renderer.rs:101-149
                                                capi.as_ptr(self.accumulators, C.c_float) if want_accumulators else None,
                                                capi.as_ptr(self.pixels, C.c_float), capi.as_ptr(self.sample_counts, C.c_uint32)))
         self.stats = ctx.stats()
-        # the last round ends at the largest count: round 0 reaches min_spp, every later one `step` more (the last clipped at spp)
-        self.stats["rounds"] = 1 + -(-(int(self.sample_counts.max()) - int(min_spp)) // int(step))
+        self.stats["rounds"] = _rounds(self.sample_counts, min_spp, step)
+        return self
+
+    def render_adaptive_sharded(self, sampler=ZSobolSampler, threshold: float = 0.01, min_spp: int = 64, step: int = 64,
+                                want_accumulators: bool = True, max_slots: int = 0) -> "RendererImage":
+        """`render_adaptive` from every GPU of the communicator (tcpt_render_adaptive_sharded; tcpt_comm_init on each rank's context):
+        every rank calls this with the same arguments and runs the rounds over its image rows y % N == rank alone; ONE grouped
+        ncclReduce of the accumulators and the counts inside libtcpt hands rank 0 the frame, bitwise the one-GPU `render_adaptive` frame.
+        `pixels`, `accumulators` and `sample_counts` are filled on rank 0 only; there stats["rounds"] = rounds of the frame."""
+        r = self.renderer
+        ctx = r.args.scene.ctx
+        if not r.args.scene.built:
+            r.args.scene.build(r.args.camera)
+        p = r.params(sampler, max_slots=max_slots)
+        ap = capi.AdaptiveParams(float(threshold), int(min_spp), int(step))
+        root = ctx.comm_rank == 0
+        if root:
+            ctx.set_option("pin_host_buffers", 1)
+            self._pinned_ctx = ctx
+        ctx.check(ctx.lib.tcpt_render_adaptive_sharded(ctx.handle, C.byref(p), C.byref(ap),
+                                                       capi.as_ptr(self.accumulators, C.c_float) if (root and want_accumulators) else None,
+                                                       capi.as_ptr(self.pixels, C.c_float) if root else None,
+                                                       capi.as_ptr(self.sample_counts, C.c_uint32) if root else None))
+        self.stats = ctx.stats()
+        if root:
+            self.stats["rounds"] = _rounds(self.sample_counts, min_spp, step)
         return self
 
     def render_sharded(self, sampler=ZSobolSampler, mode: str = "tile", want_accumulators: bool = True, spp_window=None, max_slots: int = 0) -> "RendererImage":
