@@ -262,7 +262,8 @@ int tcpt_group_render_adaptive(tcpt_group* g, const tcpt_render_params* job, con
  * (Morton order + radix tree, collapsed to the 4-wide records the traversal kernels read: csrc/lbvh.cuh; the reference's O(N^2) builder is
  * a parity requirement for the config scenes only).  triangles = n_triangles x 9 floats on the host (world space = Render space, one
  * primitive with the identity transform, primitive index 0, triangle index = position in the array).  Afterwards tcpt_trace /
- * tcpt_trace_device work; tcpt_render* refuse.  tcpt_soup_build_info: device time of the build, 128-byte records, wide levels. */
+ * tcpt_trace_device work; tcpt_render* refuse.  Refused before any device work: n_triangles = 0 or option "soup_leaf" outside [1, 16]
+ * (TCPT_ERR_INVALID), n_triangles >= 2^27 - 16 (TCPT_ERR_LIMIT).  tcpt_soup_build_info: device time of the build, 128-byte records, wide levels. */
 int tcpt_scene_build_soup(tcpt_ctx* ctx, const float* triangles, uint32_t n_triangles);
 int tcpt_soup_build_info(const tcpt_ctx* ctx, double* build_ms, uint64_t* n_records, uint32_t* levels);
 

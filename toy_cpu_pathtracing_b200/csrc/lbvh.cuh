@@ -208,6 +208,7 @@ struct Built {
     float4* tri_verts = nullptr; uint64_t n_slots = 0;
     uint32_t levels = 0, max_stack = 0;
     float build_ms = 0.0f;
+    bool too_deep = false;                              // (on failure) the tree is deeper than the wide levels the build allows
 };
 
 #define LB_CU(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { err = std::string(#call) + ": " + cudaGetErrorString(e_); cleanup(); return false; } } while (0)
@@ -273,7 +274,7 @@ inline bool build(const float* d_tri9, uint32_t n, uint32_t leaf, int sm_count, 
             const uint32_t zero = 0u;
             LB_CU(cudaMemcpyAsync(d_cnt, &zero, sizeof zero, cudaMemcpyHostToDevice, s));
             std::swap(d_q0, d_q1);
-            if (levels > 64) { err = "soup: radix tree deeper than 64 wide levels"; cleanup(); return false; }
+            if (levels > 64) { out.too_deep = true; err = "soup: radix tree deeper than 64 wide levels"; cleanup(); return false; }
         }
     }
     k_roots<<<1, 32, 0, s>>>(d_nodes, d_blo, d_bhi, (int)M, n);

@@ -1136,6 +1136,9 @@ int tcpt_upload_flat_scene(tcpt_ctx* ctx, const tcpt_flat_scene* s) {
 // BASELINE.json configs[4]: a triangle soup as a traversal-only scene, BVH built on the device (csrc/lbvh.cuh)
 int tcpt_scene_build_soup(tcpt_ctx* ctx, const float* triangles, uint32_t n_triangles) {
     if (!ctx || !triangles || n_triangles == 0) return TCPT_ERR_INVALID;
+    // refused before the device is touched: the scene built before stays in place
+    if (ctx->opt.soup_leaf < 1 || ctx->opt.soup_leaf > 16) return fail(ctx, TCPT_ERR_INVALID, "build_soup: option soup_leaf must be in [1, 16]");
+    if (n_triangles >= (1u << 27) - 16u) return fail(ctx, TCPT_ERR_LIMIT, "build_soup: 2^27 - 16 triangles or more (a stack entry addresses 2^27 item slots)");
     if (!ctx->stream) return fail(ctx, TCPT_ERR_CUDA, "no CUDA device");
     CU(cudaSetDevice(ctx->device));
     // the small tables of a one-primitive scene (identity transform, Render space = world space) go through the ordinary upload ...
@@ -1163,7 +1166,7 @@ int tcpt_scene_build_soup(tcpt_ctx* ctx, const float* triangles, uint32_t n_tria
     std::string err;
     const bool ok = tcpt::lbvh::build(d_tri, n_triangles, (uint32_t)ctx->opt.soup_leaf, ctx->sm_count, ctx->stream, b, err);
     cudaFree(d_tri);
-    if (!ok) return fail(ctx, TCPT_ERR_CUDA, "build_soup: " + err);
+    if (!ok) return fail(ctx, b.too_deep ? TCPT_ERR_LIMIT : TCPT_ERR_CUDA, "build_soup: " + err);
     ctx->dev.allocs.push_back(b.nodes); ctx->dev.allocs.push_back(b.tri_verts);
     if (b.max_stack >= TCPT_TRAVERSAL_STACK) return fail(ctx, TCPT_ERR_LIMIT, "build_soup: BVH deeper than the traversal stack");
     ctx->dev.view.nodes = b.nodes; ctx->dev.view.tri_verts = b.tri_verts;
